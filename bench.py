@@ -2,7 +2,10 @@
 """Benchmark of the P-Companion hot path on B200 (contract: see the task statement / DESIGN.md section 6).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload all|gat|gat_skewed|retrieval|retrieval_dense|pcompanion|c1|c5]
+                    [--workload all|gat|gat_skewed|retrieval|retrieval_dense|pcompanion|c1|c5] [--dump-outputs DIR]
+
+Every timed region is exactly K steps.  With the same arguments every run draws the same inputs, so two builds can be
+compared output for output with --dump-outputs.
 
 BASELINE.json's metric has two halves - "GAT edges/sec fwd+bwd (Product2Vec) & top-K queries/sec at 1/2/4/8 B200" -
 so the default run (`--workload all`) measures both and prints ONE JSON line on rank 0:
@@ -39,7 +42,6 @@ EDGES_PER_GPU = 20_000_000
 TRIPLETS = 131_072
 KNEG = 5
 SEED = 1234
-SHORT_LEG_SECONDS = 0.4      # sub-records whose step is a few ms are timed over at least this long (a multiple of --steps)
 FP64_TFLOPS_NOMINAL = 37.0   # B200 vector fp64 (HGX B200: 296 TFLOP/s per 8 GPUs); no measured figure in MEASURED_PEAKS.json
 
 # SURVEY.md 8(d): algorithmic bytes of the three sparse kernels (fp32, per edge / per node)
@@ -161,7 +163,40 @@ def warm_up(fn, min_steps, min_seconds, dev, world):
         torch.cuda.synchronize()
 
 
-def _time_once(fn, steps, dev, world, flush):
+class TrainingState:
+    """A copy of what a training step reads and changes - parameters and buffers, optimiser state and torch's CPU generator
+    (it draws the dropout seeds) - that restore() writes back in place.  Taken after exactly --warmup steps and restored
+    after the time-based part of the warm-up, so the timed steps compute the same numbers in every run with the same
+    arguments, however many steps the clocks needed."""
+
+    def __init__(self, model, opt):
+        self.live = list(model.state_dict().values()) + [v for s in opt.state.values() for v in s.values() if torch.is_tensor(v)]
+        self.saved = [t.clone() for t in self.live]
+        self.rng = torch.get_rng_state()
+
+    def restore(self):
+        with torch.no_grad():
+            for t, s in zip(self.live, self.saved):
+                t.copy_(s)
+        torch.set_rng_state(self.rng)
+        torch.cuda.synchronize()
+
+
+def dump_outputs(args, prefix, arrays):
+    """--dump-outputs DIR: every array as DIR/<prefix>.<name>.npy; floating point keeps float64 or becomes float32,
+    integers become float64 (exact for indices below 2**53)."""
+    import numpy as np
+    os.makedirs(args.dump_outputs, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if torch.is_tensor(a) else np.asarray(a)
+        a = a.astype(np.float32 if a.dtype.kind == "f" and a.dtype != np.float64 else np.float64)
+        np.save(os.path.join(args.dump_outputs, f"{prefix}.{name}.npy"), a)
+
+
+def timed_steps(fn, steps, dev, world, flush=None):
+    """Average device time of exactly `steps` calls of fn (CUDA events on the current stream, barrier + synchronize on both
+    sides, max over ranks) and fn's result of the last call.  With `flush` every step is timed on its own and the L2 flush
+    between the steps is not."""
     torch.cuda.synchronize()
     if world > 1:
         _dist().barrier()
@@ -186,19 +221,6 @@ def _time_once(fn, steps, dev, world, flush):
     if world > 1:
         _dist().barrier()
     return max_over_ranks([ms], dev, world)[0], out
-
-
-def timed_steps(fn, steps, dev, world, flush=None, min_seconds=0.0):
-    """Average device time of `steps` calls of fn (CUDA events on the current stream, barrier + synchronize on both sides,
-    max over ranks).  With `flush` every step is timed on its own and the L2 flush between the steps is not.
-    min_seconds (legs whose step is a few milliseconds): when the K steps took less than that, the measurement is repeated
-    with a multiple of K steps that fills it - a single stall of the clock sampler's nvidia-smi poll (tens of ms) would
-    otherwise double a 30 ms region.  The step count is derived from the max-over-ranks time: the same on every rank."""
-    ms, out = _time_once(fn, steps, dev, world, flush)
-    if min_seconds > 0.0 and ms * steps < min_seconds * 1e3:
-        reps = min(int(math.ceil(min_seconds * 1e3 / max(ms * steps, 1e-3))), 200)
-        ms, out = _time_once(fn, steps * reps, dev, world, flush)
-    return ms, out
 
 
 # ============================================================================= GAT leg, one GPU (C2)
@@ -228,12 +250,14 @@ def gat_single(args, dev):
     trip_host = trip.cpu().pin_memory()
     loss_host = torch.empty((), dtype=torch.float32).pin_memory()
 
-    def step(x, tr):
+    def step(x, tr, keep=None):
         emb = model.forward_graph(x, graph)
         loss = model.triplet_loss_indexed(emb, tr[:, 0], tr[:, 1], tr[:, 2:])
         opt.zero_grad(set_to_none=True)
         loss.backward()
         opt.step()
+        if keep is not None:
+            keep["embeddings"] = emb.detach()
         return loss
 
     # end-to-end leg: every step's inputs come from pinned host memory.  The copy of step i+1 is issued on a
@@ -259,17 +283,22 @@ def gat_single(args, dev):
             loss = step(xs, ts)
             loss_host.copy_(loss.detach(), non_blocking=True)
 
-    warm_up(lambda: step(x_dev, trip), args.warmup, 0.5, dev, 1)
+    for _ in range(args.warmup):
+        step(x_dev, trip)
+    start = TrainingState(model, opt)
+    warm_up(lambda: step(x_dev, trip), 1, 0.5, dev, 1)
+    start.restore()
 
     # ---- device-resident timed region (per-kernel events on the launching stream)
     sampler.mark()
     _lib.PROFILE = []
     launches0 = _lib.LAUNCHES
+    last = {} if args.dump_outputs else None
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     torch.cuda.synchronize()
     ev0.record()
-    for _ in range(args.steps):
-        loss = step(x_dev, trip)
+    for i in range(args.steps):
+        loss = step(x_dev, trip, last if i == args.steps - 1 else None)
     ev1.record()
     torch.cuda.synchronize()
     total_ms = ev0.elapsed_time(ev1)
@@ -277,6 +306,14 @@ def gat_single(args, dev):
     launches = _lib.LAUNCHES - launches0
     clocks = sampler.stop()
     ms_per_step = total_ms / args.steps
+    if args.dump_outputs:
+        # the step's loss, the updated parameters / BatchNorm statistics, the gradients, and a fixed sample of the
+        # embedding rows (all n x 128 of them would be 512 MB)
+        rows = torch.randperm(n, generator=torch.Generator().manual_seed(SEED))[:8192].sort().values
+        dump_outputs(args, "gat", {"loss": loss, "embedding_rows": rows, "embeddings": last["embeddings"][rows.to(dev)],
+                                   **{"state." + k: v for k, v in model.state_dict().items()},
+                                   **{"grad." + k: p.grad for k, p in model.named_parameters() if p.grad is not None}})
+        del last
 
     per_kernel = {}
     for name, s, t in prof:
@@ -610,11 +647,11 @@ def pcompanion_leg(args, rank, world, dev, batch, cpu=False):
     warm_up(lambda: step(bt_dev), args.warmup, 1.0, dev, world)
     sampler.mark()
     l0 = _lib.LAUNCHES
-    ms, _ = timed_steps(lambda: step(bt_dev), args.steps, dev, world, flush, SHORT_LEG_SECONDS)
+    ms, _ = timed_steps(lambda: step(bt_dev), args.steps, dev, world, flush)
     launches = _lib.LAUNCHES - l0
     clocks = sampler.stop()
     step_e2e()
-    e2e_ms, _ = timed_steps(step_e2e, args.steps, dev, world, flush, SHORT_LEG_SECONDS)
+    e2e_ms, _ = timed_steps(step_e2e, args.steps, dev, world, flush)
     eager = None
     if small and world == 1:
         # launch-bound regime: the whole step (forward + loss + backward + Adam) captured once in a CUDA graph and replayed
@@ -625,12 +662,12 @@ def pcompanion_leg(args, rank, world, dev, batch, cpu=False):
         launches = (_lib.LAUNCHES - l1) // 4 * args.steps                # C-ABI calls inside one replay x timed replays
         for _ in range(args.warmup):
             gstep(bt_dev)
-        ms, _ = timed_steps(lambda: gstep(bt_dev), args.steps, dev, world, flush, SHORT_LEG_SECONDS)
+        ms, _ = timed_steps(lambda: gstep(bt_dev), args.steps, dev, world, flush)
 
         def gstep_e2e():
             loss_host.copy_(gstep(host).detach(), non_blocking=True)
         gstep_e2e()
-        e2e_ms, _ = timed_steps(gstep_e2e, args.steps, dev, world, flush, SHORT_LEG_SECONDS)
+        e2e_ms, _ = timed_steps(gstep_e2e, args.steps, dev, world, flush)
     if rank != 0:
         return None
     peak, peak_src = measured_peaks()
@@ -652,7 +689,7 @@ def pcompanion_leg(args, rank, world, dev, batch, cpu=False):
                          "note": "whole step against the [B,T] similarity write, the type-table read / gradient / Adam traffic "
                                  "and the per-sample rows; small batches are launch-latency bound, not bandwidth bound"},
             "cpu_baseline": cpu_baseline_pcompanion(cfg, b) if cpu else None, "clocks": clocks,
-            "cuda_graph": eager is not None, "eager": eager, "min_timed_seconds": SHORT_LEG_SECONDS,
+            "cuda_graph": eager is not None, "eager": eager,
             "e2e": {"value": b * world / (e2e_ms * 1e-3), "unit": "samples/s", "ms_per_step": e2e_ms,
                     "h2d_bytes_per_step": sum(v.numel() * v.element_size() for v in host.values()) * world,
                     "d2h_bytes_per_step": 4 * world},
@@ -730,11 +767,13 @@ def retrieval_leg(args, rank, world, dev, dense=False, cpu=False):
     warm_up(step, args.warmup, 1.5, dev, world)
     sampler.mark()
     launches0 = _lib.LAUNCHES
-    ms, _ = timed_steps(step, args.steps, dev, world, None, SHORT_LEG_SECONDS)
+    ms, (scores, idx) = timed_steps(step, args.steps, dev, world)
     launches = _lib.LAUNCHES - launches0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args, "retrieval_dense" if dense else "retrieval", {"scores": scores, "indices": idx})
     step_e2e()
-    e2e_ms, _ = timed_steps(step_e2e, args.steps, dev, world, None, SHORT_LEG_SECONDS)
+    e2e_ms, _ = timed_steps(step_e2e, args.steps, dev, world)
     # per-kernel device time from a separate profiled pass (CUDA events around every C-ABI call)
     _lib.PROFILE = []
     for _ in range(args.steps):
@@ -784,7 +823,6 @@ def retrieval_leg(args, rank, world, dev, dense=False, cpu=False):
                                    "fused candidate top-K + exact fp64 re-scoring" if dense else "type-segmented exact fp64 scoring "
                                    "(device-side grouping), per-shard lists all-gathered and merged"),
                        "l2": "the catalog (5.12 GB per 10M rows) exceeds the 126 MB L2; no flush needed"},
-            "min_timed_seconds": SHORT_LEG_SECONDS,
             "roofline": roofline, "abi_ms_per_step": {n_: round(v, 4) for n_, v in sorted(per_call.items(), key=lambda kv: -kv[1])},
             "cpu_baseline": cpu_baseline_retrieval() if cpu else None,
             "clocks": clocks,
@@ -1159,9 +1197,19 @@ def main():
     ap.add_argument("--queries", type=int, default=4096)
     ap.add_argument("--skip-cpu", action="store_true", help="skip the CPU-baseline legs (profiling runs)")
     ap.add_argument("--dense", action="store_true", help="(compat) with --workload retrieval: same as --workload retrieval_dense")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy: the C2 training "
+                         "step (gat.*: loss, updated parameters and BatchNorm statistics, gradients, a fixed sample of the "
+                         "embedding rows) and the top-K results (retrieval.*, retrieval_dense.*); one GPU only.  The "
+                         "P-Companion, skewed-graph and C1 legs of --workload all are timed but not dumped")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.dense and args.workload == "retrieval":
         args.workload = "retrieval_dense"
+    if args.dump_outputs and (args.impl != "ours" or args.gpus != 1 or int(os.environ.get("WORLD_SIZE", 1)) != 1
+                              or args.workload not in ("all", "gat", "retrieval", "retrieval_dense")):
+        ap.error("--dump-outputs needs --impl ours on one GPU and --workload all, gat, retrieval or retrieval_dense")
     if args.impl == "ours":
         args.warmup = max(args.warmup, 3)      # timing rule: at least 3 untimed warm-up steps (reported as run)
     if args.impl == "reference":

@@ -46,3 +46,16 @@ def state_dict_from(g, prefix="sd/", dtype=None):
     if dtype is not None:
         out = {k: (v.astype(dtype) if np.issubdtype(v.dtype, np.floating) else v) for k, v in out.items()}
     return out
+
+
+def golden_grad(g, name, grad):
+    """(grad, golden gradient of parameter `name`).  A fixture may store a weight matrix's gradient as every
+    g["grad_stride"]-th element of the flattened matrix (keeps the file small); `grad` is then sampled the same way.
+    The stride is coprime with the row lengths, so every row and every column of the matrix is compared."""
+    ref = g["grad/" + name]
+    if tuple(ref.shape) == tuple(grad.shape):
+        return grad, ref
+    stride, numel = int(g["grad_stride"]), grad.reshape(-1).shape[0]
+    assert grad.ndim > 1 and ref.ndim == 1 and ref.size == -(-numel // stride), \
+        f"grad {name}: shape {tuple(grad.shape)} is neither the stored {ref.shape} nor a matrix it was sampled from"
+    return grad.reshape(-1)[::stride], ref

@@ -1,18 +1,19 @@
 #!/usr/bin/env python
 """Generate the golden fixtures in tests/golden/ by running the REAL reference.
 
-Run in the build container only (needs /root/reference):
+Needs a checkout of the reference project:
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <path to the reference checkout>
 
-The reference is imported from a throw-away copy under /tmp (its Config() mkdirs next to its
+The reference is imported from a throw-away temporary copy (its Config() mkdirs next to its
 own sources, and Python would write __pycache__ there).  Config() is never instantiated; a
 duck-typed namespace with the same attributes is used instead.  Seeds: random.seed(0),
 torch.manual_seed(0), PYTHONHASHSEED irrelevant (every set is sorted before it is stored).
 
 Fixtures (all float32 / int, a few hundred KB in total):
   p2v_module.npz  Product2Vec state_dict + inputs -> eval / train forward, BN running stats,
-                  triplet loss and every parameter gradient (DROPOUT=0).
+                  triplet loss and every parameter gradient (DROPOUT=0); weight-matrix gradients
+                  as every GRAD_STRIDE-th element of the flattened matrix (tests/conftest.py golden_grad).
   p2v_graph.npz   small BPG + features -> generate_all_embeddings().
   bpg_c1.npz      the default synthetic BPG (config C1): edge sets, similarity /
                   complementary pairs, set helpers, neighbour samples, types.
@@ -30,15 +31,15 @@ import numpy as np
 import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF_SRC = "/root/reference"
+GRAD_STRIDE = 7   # coprime with every row length (128, 256): the sample covers every row and column
 
 
-def import_reference():
+def import_reference(ref_src):
     tmp = tempfile.mkdtemp(prefix="pc_ref_")
     dst = os.path.join(tmp, "ref")
     def skip(d, names):  # top-level models/ holds only checkpoints; src/models is needed
-        return [n for n in names if n in (".git", "__pycache__") or (d == REF_SRC and n == "models")]
-    shutil.copytree(REF_SRC, dst, ignore=skip)
+        return [n for n in names if n in (".git", "__pycache__") or (d == ref_src and n == "models")]
+    shutil.copytree(ref_src, dst, ignore=skip)
     sys.path.insert(0, dst)
     sys.dont_write_bytecode = True
     return dst
@@ -95,7 +96,9 @@ def golden_p2v_module():
     out["train_negative_emb"] = n.detach().numpy()
     out["train_loss"] = loss.detach().numpy()
     for k, v in m.named_parameters():
-        out["grad/" + k] = v.grad.numpy().copy()
+        gk = v.grad.numpy()
+        out["grad/" + k] = gk.reshape(-1)[::GRAD_STRIDE].copy() if gk.ndim > 1 else gk.copy()
+    out["grad_stride"] = np.array(GRAD_STRIDE, np.int64)
     out["train_running_mean"] = m.ffn[1].running_mean.numpy().copy()
     out["train_running_var"] = m.ffn[1].running_var.numpy().copy()
     out["train_num_batches_tracked"] = m.ffn[1].num_batches_tracked.numpy().copy()
@@ -264,7 +267,7 @@ def golden_metrics():
 
 
 if __name__ == "__main__":
-    import_reference()
+    import_reference(os.path.abspath(sys.argv[1]))
     golden_p2v_module()
     golden_p2v_graph()
     golden_bpg_c1()

@@ -153,15 +153,21 @@ def test_similarity_dataset_requires_pairs_like_reference():
         SimilarityDataset(b, make_cfg())
 
 
-REF_CKPT = "/root/reference/models/run_20241206_210422/product2vec.pth"
-
-
-@pytest.mark.skipif(not os.path.exists(REF_CKPT), reason="the reference checkout (with its shipped checkpoints) is not on this box")
-def test_shipped_reference_checkpoint_loads_into_the_drop_in_modules():
-    """scripts/pretrain_product2vec.py:44-49 layout {'model_state_dict', 'embeddings', 'type_to_idx'}: the state_dict loads
-    strictly into Product2Vec, the embedding dict feeds PCompanion.__init__ as train.py:42-43 does."""
+def test_checkpoint_in_reference_layout_loads_into_the_drop_in_modules(tmp_path):
+    """A checkpoint written in the layout of the reference's product2vec.pth (scripts/pretrain_product2vec.py:44-49:
+    {'model_state_dict', 'embeddings', 'type_to_idx'}), filled from p2v_graph.npz: the real reference's state_dict, the
+    embedding dict its generate_all_embeddings() returned for that model, and the graph's product types.  The
+    state_dict loads strictly into Product2Vec, the embedding dict feeds PCompanion.__init__ as train.py:42-43 does."""
     from pcompanion_b200 import PCompanion, Product2Vec
-    ck = torch.load(REF_CKPT, map_location="cpu", weights_only=True)
+    g = load_golden("p2v_graph.npz")
+    n = g["embeddings"].shape[0]
+    ids = [f"P{str(i).zfill(6)}" for i in range(n)]
+    types = sorted({f"type_{i % 5}" for i in range(n)})                 # node types of the golden graph (make_golden.py)
+    path = tmp_path / "product2vec.pth"
+    torch.save({"model_state_dict": {k: torch.tensor(v) for k, v in state_dict_from(g).items()},
+                "embeddings": {p: torch.tensor(e) for p, e in zip(ids, g["embeddings"])},
+                "type_to_idx": {t: i for i, t in enumerate(types)}}, path)
+    ck = torch.load(path, map_location="cpu", weights_only=True)
     m = Product2Vec(make_cfg())
     missing = m.load_state_dict(ck["model_state_dict"], strict=True)
     assert not missing.missing_keys and not missing.unexpected_keys

@@ -10,7 +10,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import load_golden, state_dict_from
+from conftest import golden_grad, load_golden, state_dict_from
 
 pytestmark = pytest.mark.gpu
 
@@ -355,7 +355,7 @@ def test_product2vec_train_step_matches_reference_golden():
     close(n, g["train_negative_emb"], what="negative")
     close(loss, g["train_loss"], what="loss")
     for k, v in m.named_parameters():
-        close(v.grad, g["grad/" + k], rel=REL_VS_FP32, atol=1e-7, what="grad " + k)   # reference grads are themselves fp32
+        close(*golden_grad(g, k, v.grad), rel=REL_VS_FP32, atol=1e-7, what="grad " + k)   # reference grads are themselves fp32
     close(m.ffn[1].running_mean, g["train_running_mean"], what="running_mean")
     close(m.ffn[1].running_var, g["train_running_var"], what="running_var")
     assert int(m.ffn[1].num_batches_tracked) == int(g["train_num_batches_tracked"])

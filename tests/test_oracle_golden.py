@@ -6,7 +6,7 @@ inputs, so agreement is limited by the reference's own rounding (~1e-6 relative)
 import numpy as np
 import torch
 
-from conftest import load_golden, state_dict_from
+from conftest import golden_grad, load_golden, state_dict_from
 from oracle import bpg as obpg
 from oracle import p2v, pcomp, retrieval, torch_port
 
@@ -222,7 +222,7 @@ def test_torch_port_state_dict_and_numbers_match_reference():
     loss.backward()
     close(loss.item(), g["train_loss"], 1e-5, 1e-6)
     for k, v in m.named_parameters():
-        close(v.grad.numpy(), g["grad/" + k], 1e-4, 1e-6)
+        close(*golden_grad(g, k, v.grad.numpy()), 1e-4, 1e-6)
     gp = load_golden("pcomp.npz")
     sdp = {k: torch.tensor(v) for k, v in state_dict_from(gp).items()}
     pm = torch_port.PortPCompanion(torch_port.default_config(DROPOUT=0.0, NUM_TYPES=40), sdp["product_embeddings.weight"])
