@@ -208,11 +208,19 @@ int pc_sample_negatives(const int32_t* anchor, const int64_t* sim_rowptr, const 
  * products of float32 values are exact in float64, so the value is fully defined; oracle/retrieval.py
  * mirrors it); ranking = (score desc, index asc); padding = (-inf, -1).
  *
+ * pc_topk_groups, pc_topk_by_type, pc_topk_rows and pc_topk_merge accept 1 <= k <= PC_TOPK_MAX_K.  k <= 32
+ * runs a warp-distributed sorted list (one entry per lane); a larger k runs a selection whose candidates are
+ * appended to shared-memory buffers with atomics and compacted by sorting.  The append order therefore varies
+ * from run to run, but (score, index) is a strict total order and the scores are exactly defined, so any exact
+ * selection returns the same entries in the same order: results are bit-for-bit reproducible for every k.
+ *
  * pc_topk_groups: score rows are processed in groups of at most 8 that rank the same contiguous run
  * members[seg_begin[g] .. seg_end[g]) of catalog row ids (the members of one complementary type in a
  * type-sorted permutation from pc_sort_keys; members == NULL means the identity, i.e. a slice of the
  * catalog).  Group g holds the rows row_ids[grp_begin[g] .. grp_begin[g+1]).  A catalog row is read
- * once per group.  k <= 32, dim % 32 == 0.  Results land at the original row positions. */
+ * once per group (for k > 32, once per sub-batch of the group's rows whose candidate buffers fit in shared
+ * memory: 8 rows up to k = 256 at dim 128).  dim % 16 == 0, dim <= 1024.  Results land at the original row positions. */
+#define PC_TOPK_MAX_K 1024
 size_t pc_topk_groups_workspace_bytes(int64_t rows, int k, int splits);
 int pc_topk_groups(const float* q, int64_t rows, int dim, const float* catalog, const int32_t* members,
                    const int32_t* row_ids, const int32_t* grp_begin, const int64_t* seg_begin, const int64_t* seg_end,
@@ -223,7 +231,8 @@ int pc_topk_groups(const float* q, int64_t rows, int dim, const float* catalog, 
  * type 0, i.e. pass n_types = 1 and type_offsets = {0, P} for an unrestricted ranking); a row_type outside
  * [0, n_types) gives an all-padding row, as `if not type_products: continue` of inference.py:97-98.  Internally:
  * keys type << 32 | row, stable radix sort on the type bytes (pc_sort_keys), one pass that marks every eighth
- * row of a type's run as the start of a group, then the pc_topk_groups kernel with one CTA row per position. */
+ * row of a type's run as the start of a group (for k > 32: every row count the large-k kernel ranks in one
+ * pass), then the pc_topk_groups kernel with one CTA row per position. */
 size_t pc_topk_by_type_workspace_bytes(int64_t rows, int k, int splits);
 int pc_topk_by_type(const float* q, int64_t rows, int dim, const float* catalog, const int32_t* members,
                     const int64_t* type_offsets, int n_types, const int32_t* row_type, int k, int splits,

@@ -17,6 +17,7 @@ from typing import Any, Dict, List, Optional, Sequence
 import torch
 
 from .bpg import BehaviorProductGraph
+from .ops import TOPK_MAX_K
 from .p_companion import PCompanion
 from .retrieval import CatalogIndex
 
@@ -59,6 +60,10 @@ class PCompanionInference:
         return {"query_ids": list(query_ids), "query_types": types}
 
     def recommend_batch(self, query_ids: Sequence[str], num_recommendations: int = 10) -> List[Dict[str, Any]]:
+        """Up to num_recommendations (1 .. TOPK_MAX_K = 1024) products per predicted complementary type; a type with
+        fewer products returns all of them, as the reference's min(k, len(type_products))."""
+        if not 1 <= num_recommendations <= TOPK_MAX_K:
+            raise ValueError(f"num_recommendations={num_recommendations} outside [1, {TOPK_MAX_K}]")
         with torch.no_grad():
             outputs = self.model(self._prepare_input(query_ids))
             comp_types = outputs["complementary_types"]                      # [B, Kt]

@@ -769,14 +769,25 @@ def type_scores_topk(base: torch.Tensor, weight: torch.Tensor, k: int, materiali
 
 # --------------------------------------------------------------------------- retrieval
 TOPK_GROUP_ROWS = 8   # score rows the kernel ranks per pass over a segment (csrc/retrieval.cu RB)
+TOPK_MAX_K = 1024     # PC_TOPK_MAX_K: the largest k the top-k kernels select
+TOPK_WARP_K = 32      # k above this runs the buffered large-k selection (csrc/retrieval.cu WARP_K)
+SPLIT_WS_BYTES = 256 << 20   # bound on the [rows, splits, k] (f64, i64) split lists chosen automatically for k > 32
 
 
-def _auto_splits(units: int, avg_len: float) -> int:
+def _check_k(k: int, what: str) -> None:
+    if not 1 <= k <= TOPK_MAX_K:
+        raise ValueError(f"{what}: k={k} outside [1, {TOPK_MAX_K}]")
+
+
+def _auto_splits(units: int, avg_len: float, k: int = 1, rows: int = 0) -> int:
     sms = 148
     if units >= 2 * sms:
         return 1
     want = max(1, (2 * sms + units - 1) // max(units, 1))
     cap = max(1, int(avg_len // 256))
+    if k > TOPK_WARP_K:
+        # every split returns k entries per row: a split must rank many more than k products, and the lists stay bounded
+        cap = min(cap, max(1, int(avg_len // (16 * k))), max(1, SPLIT_WS_BYTES // max(1, rows * k * 16)))
     return max(1, min(want, cap, 1024))
 
 
@@ -784,6 +795,7 @@ def topk_segments(q: torch.Tensor, catalog: torch.Tensor, seg_begin: torch.Tenso
                   members: Optional[torch.Tensor] = None, index_base: int = 0, splits: Optional[int] = None):
     """Exact top-k of every row over its run of catalog rows; returns (scores f64 [R,k], idx i64 [R,k]).
     Rows that rank the same run (same complementary type) are grouped, eight per pass (pc_topk_groups)."""
+    _check_k(k, "topk_segments")
     rows, dim = q.shape
     dev_ = q.device
     out_s = torch.empty(rows, k, dtype=F64, device=dev_)
@@ -806,7 +818,7 @@ def topk_segments(q: torch.Tensor, catalog: torch.Tensor, seg_begin: torch.Tenso
     g_end = seg_end[order][starts].contiguous()
     row_ids = order.to(I32).contiguous()
     if splits is None:
-        splits = _auto_splits(n_groups, float((g_end - g_beg).float().mean().item()))
+        splits = _auto_splits(n_groups, float((g_end - g_beg).float().mean().item()), k, rows)
     ws = _lib.workspace(_lib.LIB.pc_topk_groups_workspace_bytes(rows, k, splits), dev_)
     call("pc_topk_groups", dev(q.contiguous(), F32, "q"), rows, dim, dev(catalog, F32, "catalog"),
          dev(members, I32, "members"), dev(row_ids, I32, "row_ids"), dev(grp_begin, I32, "grp_begin"),
@@ -820,6 +832,7 @@ def topk_by_type(q: torch.Tensor, catalog: torch.Tensor, type_offsets: torch.Ten
                  splits: Optional[int] = None):
     """Exact top-k of every row over the catalog rows of its type, grouping done on the device (pc_topk_by_type): no
     host synchronisation between the inputs and the result.  Returns (scores f64 [R,k], idx i64 [R,k])."""
+    _check_k(k, "topk_by_type")
     q = q.contiguous()
     rows, dim = q.shape
     out_s = torch.empty(rows, k, dtype=F64, device=q.device)
@@ -830,7 +843,7 @@ def topk_by_type(q: torch.Tensor, catalog: torch.Tensor, type_offsets: torch.Ten
         # expected number of groups without looking at the data: distinct types hit + one more group per 8 rows
         n_cat = members.numel() if members is not None else catalog.shape[0]
         distinct = n_types * (1.0 - math.exp(-rows / max(n_types, 1)))
-        splits = _auto_splits(int(distinct + rows / TOPK_GROUP_ROWS) + 1, n_cat / max(n_types, 1))
+        splits = _auto_splits(int(distinct + rows / TOPK_GROUP_ROWS) + 1, n_cat / max(n_types, 1), k, rows)
     ws = _lib.workspace(_lib.LIB.pc_topk_by_type_workspace_bytes(rows, k, splits), q.device)
     call("pc_topk_by_type", dev(q, F32, "q"), rows, dim, dev(catalog, F32, "catalog"), dev(members, I32, "members"),
          dev(type_offsets, I64, "type_offsets"), int(n_types), dev(row_type, I32, "row_type"), k, splits, int(index_base),
@@ -865,11 +878,13 @@ def score_topk_dense(q: torch.Tensor, catalog: torch.Tensor, k: int, type_id: Op
 
 
 def topk_rows(values: torch.Tensor, k: int, splits: Optional[int] = None):
-    """Row-wise top-k of a materialised fp32 matrix, ties -> lowest index (torch.topk replacement)."""
+    """Row-wise top-k of a materialised fp32 matrix, ties -> lowest index (torch.topk replacement).  Columns past the
+    end pad with (-inf, -1) when cols < k."""
+    _check_k(k, "topk_rows")
     values = values.contiguous()
     rows, cols = values.shape
     if splits is None:
-        splits = _auto_splits(rows, float(cols))
+        splits = _auto_splits(rows, float(cols), k, rows)
     out_s = torch.empty(rows, k, dtype=F64, device=values.device)
     out_i = torch.empty(rows, k, dtype=I64, device=values.device)
     ws = _lib.workspace(_lib.LIB.pc_topk_rows_workspace_bytes(rows, k, splits), values.device)
@@ -880,6 +895,7 @@ def topk_rows(values: torch.Tensor, k: int, splits: Optional[int] = None):
 
 def topk_merge(scores: torch.Tensor, idx: torch.Tensor, k: int):
     """Merge [R, lists*k] candidates -> [R, k] (per-shard merge, SURVEY 8e)."""
+    _check_k(k, "topk_merge")
     rows, total = scores.shape
     lists = total // k
     out_s = torch.empty(rows, k, dtype=F64, device=scores.device)

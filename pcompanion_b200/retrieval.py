@@ -30,10 +30,9 @@ def _score_matrix(rows: torch.Tensor, targets: torch.Tensor) -> torch.Tensor:
 class Metrics:
     @staticmethod
     def hit_at_k(predictions: torch.Tensor, ground_truth: torch.Tensor, k: int) -> float:
-        """metrics.py:7-26."""
+        """metrics.py:7-26.  k is clipped to the number of columns as torch.topk requires; after that, k may be up to
+        ops.TOPK_MAX_K (ValueError beyond)."""
         k = min(k, predictions.size(1))
-        if k > 32:
-            raise ValueError("hit_at_k: k > 32 is not supported by the warp top-k kernel")
         _, top_k = ops.topk_rows(predictions.float(), k)
         hits = torch.any(top_k == ground_truth.unsqueeze(1), dim=1)
         return hits.float().mean().item()
@@ -102,9 +101,9 @@ class CatalogIndex:
 
     def topk(self, queries: torch.Tensor, k: int, row_type: Optional[torch.Tensor] = None,
              splits: Optional[int] = None) -> Tuple[torch.Tensor, torch.Tensor]:
-        """Top-k per query row; row_type[r] restricts row r to products of that type (all products
-        when row_type is None).  Returns (scores float64 [R, k], global indices int64 [R, k]),
-        padded with (-inf, -1) when a type has fewer than k products."""
+        """Top-k per query row, 1 <= k <= ops.TOPK_MAX_K (1024; ValueError otherwise); row_type[r] restricts row r
+        to products of that type (all products when row_type is None).  Returns (scores float64 [R, k], global
+        indices int64 [R, k]), padded with (-inf, -1) when a type has fewer than k products."""
         queries = queries.contiguous().float()
         if row_type is None:
             if self._all is None:
@@ -132,7 +131,8 @@ class CatalogIndex:
 
     def recommend(self, projected_embeddings: torch.Tensor, complementary_types: torch.Tensor, k: int = 10):
         """The loop of inference.py:93-113 for a whole batch: projected [B, Kt, D], types [B, Kt] ->
-        (scores [B, Kt, k], product indices [B, Kt, k])."""
+        (scores [B, Kt, k], product indices [B, Kt, k]), 1 <= k <= ops.TOPK_MAX_K; a type with fewer than k products
+        pads its rows with (-inf, -1)."""
         b, kt, d = projected_embeddings.shape
         s, i = self.topk(projected_embeddings.reshape(b * kt, d), k, complementary_types.reshape(-1))
         return s.reshape(b, kt, k), i.reshape(b, kt, k)
