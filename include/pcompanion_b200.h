@@ -238,6 +238,21 @@ int pc_topk_by_type(const float* q, int64_t rows, int dim, const float* catalog,
                     const int64_t* type_offsets, int n_types, const int32_t* row_type, int k, int splits,
                     int64_t index_base, double* out_scores, int64_t* out_idx, void* workspace, size_t workspace_bytes,
                     pc_stream_t stream);
+/* Rank of a target (the full-catalog form of hit_at_k, src/utils/metrics.py:7-26, over the per-type filter of
+ * inference.py:93-113): out_rank[r] = number of products of row r's run members[type_offsets[t] .. type_offsets[t+1])
+ * (t = row_type[r]; row_type NULL: type 0, pass n_types = 1 and type_offsets = {0, P}) whose (score, global index)
+ * ranks strictly before (score(q[r], target_rows[r]), target_idx[r]) under the ranking rule above; -1 when t is outside
+ * [0, n_types).  target_rows [rows, dim] is the target's catalog row and target_idx [rows] its global index (ties).
+ * Membership of the target in the run is not checked: the caller gives -1 to rows whose target is not a member.  For
+ * a member, 0 <= out_rank[r] < k  <=>  the target is in row r's pc_topk_by_type list for k, at position out_rank[r].
+ * The target's score is computed with the streaming pass's arithmetic, so it is the same bits.  Grouping as
+ * pc_topk_by_type (k <= 32); the counts of every split are added into out_rank (integers: deterministic), so splits
+ * need no workspace and no merge.  members, type_offsets, index_base, dim and rows < 2^31 as pc_topk_by_type. */
+size_t pc_rank_by_type_workspace_bytes(int64_t rows);
+int pc_rank_by_type(const float* q, int64_t rows, int dim, const float* catalog, const int32_t* members,
+                    const int64_t* type_offsets, int n_types, const int32_t* row_type, const float* target_rows,
+                    const int64_t* target_idx, int splits, int64_t index_base, int64_t* out_rank, void* workspace,
+                    size_t workspace_bytes, pc_stream_t stream);
 /* Dense whole-catalog variant on the tensor cores (north_star part 4): scores = Q . C^T as a TF32 tcgen05
  * GEMM (never materialised; approximate scores only select candidates), per-type mask (type_id[p] == row_type[r]; row_type NULL or < 0 = no mask) and a
  * per-row candidate list fused into the epilogue, then exact float64 re-scoring + ranking of the candidates.

@@ -714,6 +714,99 @@ int by_type_large(const float* q, int64_t rows, int dim, const float* catalog, c
   }
 }
 
+// ---- rank of a target (pc_rank_by_type).  The rank of row r's target is the number of products of the row's run that
+// rank strictly before (s*, g) = (score of the target, its global index); it needs no selection state, only a count
+// per row.  Counts are integers, so the CTAs of every split add into the zeroed out_rank in any order and the result is
+// the same: no split lists and no merge.
+__global__ void __launch_bounds__(TK_WARPS * 32, 2)
+rank_planned_kernel(const float* __restrict__ Q, int dim, const float* __restrict__ catalog,
+                    const int32_t* __restrict__ members, const int32_t* __restrict__ row_ids,
+                    const int32_t* __restrict__ grp_rows, const uint64_t* __restrict__ keys,
+                    const int64_t* __restrict__ type_offsets, int n_types, int64_t p0, const float* __restrict__ target_rows,
+                    const int64_t* __restrict__ target_idx, int splits, int64_t index_base,
+                    unsigned long long* __restrict__ out_rank) {
+  const int64_t p = p0 + blockIdx.y;
+  const int n_rows = grp_rows[p];
+  if (n_rows == 0) return;                      // uniform over the CTA
+  const int64_t t = int64_t(keys[p] >> 32);
+  if (t >= n_types) {                           // no valid type: the target can never be listed
+    if (blockIdx.x == 0 && threadIdx.x < n_rows) out_rank[row_ids[p + threadIdx.x]] = ~0ull;
+    return;
+  }
+  extern __shared__ double smem_d[];
+  double* q_s = smem_d;                                                      // [RB][dim], rows >= n_rows are zero
+  float* tiles = reinterpret_cast<float*>(q_s + RB * dim);                   // [TK_WARPS][2][BATCH][TILE_LD]
+  double* tgt_s = reinterpret_cast<double*>(tiles + TK_WARPS * 2 * TILE_FLOATS);  // [RB] target scores
+  int64_t* tgt_i = reinterpret_cast<int64_t*>(tgt_s + RB);                   // [RB] target global indices
+  unsigned long long* cnt_s = reinterpret_cast<unsigned long long*>(tgt_i + RB);  // [RB] CTA counts
+  const int lane = lane_id(), w = warp_id();
+  for (int i = threadIdx.x; i < RB * dim; i += blockDim.x) {
+    const int r = i / dim, d = i - r * dim;
+    q_s[i] = r < n_rows ? double(Q[int64_t(row_ids[p + r]) * dim + d]) : 0.0;
+  }
+  if (threadIdx.x < RB) cnt_s[threadIdx.x] = 0;
+  __syncthreads();
+  if (threadIdx.x < RB) {
+    // the arithmetic of score_pass in its order (sequential in d, fma(q, c, acc) from 0): the target's streamed score
+    // has the same bits, so the target never ranks before itself
+    const int r = threadIdx.x;
+    double acc = 0.0;
+    int64_t g = -1;
+    if (r < n_rows) {
+      const int64_t row = row_ids[p + r];
+      const float* tr = target_rows + row * dim;
+      for (int d = 0; d < dim; ++d) acc = fma(q_s[r * dim + d], double(tr[d]), acc);
+      g = target_idx[row];
+    }
+    tgt_s[r] = acc;
+    tgt_i[r] = g;
+  }
+  __syncthreads();
+  const int64_t beg = type_offsets[t], end = type_offsets[t + 1];
+  const int64_t len = end > beg ? end - beg : 0;
+  const int64_t per = (ceil_div(len, int64_t(splits)) + 31) / 32 * 32;
+  const int64_t sb = beg + per * blockIdx.x;
+  const int64_t se = min(end, sb + per);
+  float* tile = tiles + w * 2 * TILE_FLOATS;
+  auto member_at = [&](int64_t pos) -> int { return pos < se ? (members ? members[pos] : int(pos)) : -1; };
+
+  unsigned cnt[RB];
+#pragma unroll
+  for (int r = 0; r < RB; ++r) cnt[r] = 0;
+  int64_t base = sb + int64_t(w) * BATCH;
+  int cur[PP], nxt[PP];
+#pragma unroll
+  for (int pp = 0; pp < PP; ++pp) cur[pp] = member_at(base + 32 * pp + lane);
+  int buf = 0;
+  if (base < se) stage_chunk(tile, catalog, dim, 0, cur);
+  asm volatile("cp.async.commit_group;" ::: "memory");
+  while (base < se) {                           // warps advance independently: nothing shared is written in the loop
+    const int64_t next_base = base + TK_WARPS * BATCH;
+#pragma unroll
+    for (int pp = 0; pp < PP; ++pp) nxt[pp] = member_at(next_base + 32 * pp + lane);
+    double acc[PP][RB];
+    score_pass<RB>(acc, tile, buf, q_s, dim, catalog, cur, nxt, next_base < se);
+#pragma unroll
+    for (int pp = 0; pp < PP; ++pp) {
+      const int64_t gidx = int64_t(cur[pp]) + index_base;
+#pragma unroll
+      for (int r = 0; r < RB; ++r)
+        cnt[r] += (cur[pp] >= 0 && ranks_before(acc[pp][r], gidx, tgt_s[r], tgt_i[r])) ? 1u : 0u;
+    }
+    base = next_base;
+#pragma unroll
+    for (int pp = 0; pp < PP; ++pp) cur[pp] = nxt[pp];
+  }
+  asm volatile("cp.async.wait_group 0;" ::: "memory");
+#pragma unroll
+  for (int r = 0; r < RB; ++r) {
+    const unsigned c = __reduce_add_sync(FULL, cnt[r]);
+    if (lane == 0 && r < n_rows && c) atomicAdd(cnt_s + r, (unsigned long long)c);
+  }
+  __syncthreads();
+  if (threadIdx.x < n_rows && cnt_s[threadIdx.x]) atomicAdd(out_rank + row_ids[p + threadIdx.x], cnt_s[threadIdx.x]);
+}
+
 }  // namespace
 }  // namespace pc
 
@@ -825,6 +918,54 @@ extern "C" int pc_topk_by_type(const float* q, int64_t rows, int dim, const floa
     }
   }
   if (splits > 1) return pc_topk_merge(ps, pi, rows, splits, k, out_scores, out_idx, stream);
+  return PC_OK;
+}
+
+extern "C" size_t pc_rank_by_type_workspace_bytes(int64_t rows) {
+  if (rows <= 0) return 0;
+  return align_up(size_t(rows) * 8, 256) + align_up(pc_sort_keys_workspace_bytes(rows), 256) + 2 * align_up(size_t(rows) * 4, 256);
+}
+
+extern "C" int pc_rank_by_type(const float* q, int64_t rows, int dim, const float* catalog, const int32_t* members,
+                               const int64_t* type_offsets, int n_types, const int32_t* row_type, const float* target_rows,
+                               const int64_t* target_idx, int splits, int64_t index_base, int64_t* out_rank, void* workspace,
+                               size_t workspace_bytes, pc_stream_t stream) {
+  PC_REQUIRE(rows >= 0 && rows < (int64_t(1) << 31), PC_ERR_INVALID, "rank_by_type: bad row count");
+  if (rows == 0) return PC_OK;
+  PC_REQUIRE(q && catalog && type_offsets && target_rows && target_idx && out_rank && workspace, PC_ERR_INVALID,
+             "rank_by_type: null pointer");
+  PC_REQUIRE(n_types >= 1 && n_types < (1 << 30), PC_ERR_INVALID, "rank_by_type: bad n_types=%d", n_types);
+  PC_REQUIRE(dim >= DCH && dim % DCH == 0 && dim <= 1024, PC_ERR_UNSUPPORTED, "rank_by_type: dim=%d must be a multiple of %d (<= 1024)", dim, DCH);
+  PC_REQUIRE(splits >= 1 && splits <= 65535, PC_ERR_UNSUPPORTED, "rank_by_type: bad splits");
+  PC_REQUIRE(workspace_bytes >= pc_rank_by_type_workspace_bytes(rows), PC_ERR_WORKSPACE, "rank_by_type: workspace too small");
+  cudaStream_t st = as_stream(stream);
+  char* ws = reinterpret_cast<char*>(workspace);
+  uint64_t* keys = reinterpret_cast<uint64_t*>(ws);             ws += align_up(size_t(rows) * 8, 256);
+  void* sort_ws = ws;                                            const size_t sort_bytes = pc_sort_keys_workspace_bytes(rows);
+  ws += align_up(sort_bytes, 256);
+  int32_t* row_ids = reinterpret_cast<int32_t*>(ws);             ws += align_up(size_t(rows) * 4, 256);
+  int32_t* grp_rows = reinterpret_cast<int32_t*>(ws);
+  PC_CUDA(cudaMemsetAsync(out_rank, 0, size_t(rows) * sizeof(int64_t), st));
+  const unsigned tb = unsigned(ceil_div(rows, 256));
+  type_keys_kernel<<<tb, 256, 0, st>>>(row_type, rows, n_types, keys);
+  PC_LAUNCH_CHECK();
+  uint32_t mask = 0;
+  for (int b = 0; b < 4; ++b)
+    if ((uint64_t(n_types) >> (8 * b)) != 0) mask |= 1u << (4 + b);
+  if (int rc = pc_sort_keys(keys, rows, mask, sort_ws, sort_bytes, stream)) return rc;
+  topk_plan_kernel<RB><<<tb, 256, 0, st>>>(keys, rows, row_ids, grp_rows);
+  PC_LAUNCH_CHECK();
+  const size_t smem = size_t(RB) * dim * sizeof(double) + size_t(TK_WARPS) * 2 * TILE_FLOATS * sizeof(float) +
+                      size_t(RB) * (sizeof(double) + sizeof(int64_t) + sizeof(unsigned long long));
+  PC_CUDA(cudaFuncSetAttribute(rank_planned_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+  for (int64_t p0 = 0; p0 < rows; p0 += 65535) {   // gridDim.y limit
+    const int64_t np = rows - p0 < 65535 ? rows - p0 : 65535;
+    dim3 grid{unsigned(splits), unsigned(np), 1u};
+    rank_planned_kernel<<<grid, TK_WARPS * 32, smem, st>>>(q, dim, catalog, members, row_ids, grp_rows, keys, type_offsets,
+                                                           n_types, p0, target_rows, target_idx, splits, index_base,
+                                                           reinterpret_cast<unsigned long long*>(out_rank));
+    PC_LAUNCH_CHECK();
+  }
   return PC_OK;
 }
 

@@ -7,19 +7,21 @@ layout ({'complementary_types', 'recommendations', 'scores'}), same semantics as
 features, top-k) - but the shipped file cannot be imported (:7-8, :17) and feeds a batch whose keys
 do not match ``PCompanion.forward``; here the batch is built with the keys forward() consumes and the
 per-type scoring runs on the type-segmented catalog kernel (exact fp64, ties -> lowest index).
-``recommend_batch`` answers many queries in one launch.
+``recommend_batch`` answers many queries in one launch.  ``rank_targets`` / ``evaluate`` score held-out
+(query, complementary product) pairs against the whole catalog: the exact position of the true product in
+``recommend``'s ranking, and hit@k / NDCG@k / MRR from those positions for any k.
 """
 from __future__ import annotations
 
 import os
-from typing import Any, Dict, List, Optional, Sequence
+from typing import Any, Dict, List, Optional, Sequence, Tuple
 
 import torch
 
 from .bpg import BehaviorProductGraph
 from .ops import TOPK_MAX_K
 from .p_companion import PCompanion
-from .retrieval import CatalogIndex
+from .retrieval import CatalogIndex, Metrics
 
 
 class PCompanionInference:
@@ -83,3 +85,42 @@ class PCompanionInference:
 
     def recommend(self, query_id: str, num_recommendations: int = 10) -> Dict[str, Any]:
         return self.recommend_batch([query_id], num_recommendations)[0]
+
+    def rank_targets(self, query_ids: Sequence[str], target_ids: Sequence[str]) -> Tuple[torch.Tensor, torch.Tensor]:
+        """Where each held-out complementary product would land in ``recommend(query)``: (ranks int64 [B], slots int64
+        [B]).  slots[b] is the position among the predicted complementary types of the one equal to the target's type
+        (-1 when the model did not predict it); ranks[b] is the target's 0-based position in that type's full ranking
+        (CatalogIndex.rank), -1 without a slot.  recommend(query_ids[b], k) lists target_ids[b] exactly when
+        0 <= ranks[b] < k, at position ranks[b] of slot slots[b].  One batched model forward."""
+        if len(query_ids) != len(target_ids):
+            raise ValueError(f"rank_targets: {len(query_ids)} queries but {len(target_ids)} targets")
+        for t in target_ids:
+            if t not in self.bpg.nodes:
+                raise ValueError(f"Product ID {t} not found in BPG")
+        batch = self._prepare_input(query_ids)
+        tgt = torch.tensor([self.bpg._index[t] for t in target_ids], dtype=torch.int64)
+        tgt_type = self._type_of[tgt].to(self.device, torch.int64)
+        tgt = tgt.to(self.device)
+        ranks = torch.full((len(query_ids),), -1, dtype=torch.int64, device=self.device)
+        if not len(query_ids):
+            return ranks, ranks.clone()
+        with torch.no_grad():
+            outputs = self.model(batch)
+            match = outputs["complementary_types"].to(torch.int64) == tgt_type[:, None]          # [B, Kt]
+            slots = torch.where(match.any(1), match.int().argmax(1).to(torch.int64), torch.full_like(tgt, -1))
+            sel = torch.nonzero(slots >= 0).squeeze(1)
+            if sel.numel():
+                queries = outputs["projected_embeddings"][sel, slots[sel]]
+                ranks[sel] = self.catalog.rank(queries, tgt[sel], tgt_type[sel])
+        return ranks, slots
+
+    def evaluate(self, query_ids: Sequence[str], target_ids: Sequence[str],
+                 ks: Sequence[int] = (1, 3, 10, 50, 100)) -> Dict[str, float]:
+        """Full-catalog retrieval quality on held-out (query, complementary product) pairs: Metrics.rank_metrics of
+        rank_targets (hit@k, ndcg@k, mrr, num_rows; a pair whose target type was not predicted is a miss) and
+        type_recall, the fraction of pairs whose target type is among the predicted complementary types.  hit@k is
+        the fraction of pairs for which recommend(query, k) lists the target."""
+        ranks, slots = self.rank_targets(query_ids, target_ids)
+        metrics = Metrics.rank_metrics(ranks, ks)
+        metrics["type_recall"] = (slots >= 0).double().mean().item() if slots.numel() else 0.0
+        return metrics

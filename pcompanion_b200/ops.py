@@ -851,6 +851,38 @@ def topk_by_type(q: torch.Tensor, catalog: torch.Tensor, type_offsets: torch.Ten
     return out_s, out_i
 
 
+def rank_by_type(q: torch.Tensor, catalog: torch.Tensor, type_offsets: torch.Tensor, n_types: int,
+                 row_type: Optional[torch.Tensor], target_rows: torch.Tensor, target_idx: torch.Tensor,
+                 members: Optional[torch.Tensor] = None, index_base: int = 0, splits: Optional[int] = None) -> torch.Tensor:
+    """Rank of each row's target among the catalog rows of the row's type (pc_rank_by_type): the number of products
+    whose (score, global index) ranks strictly before (q[r] . target_rows[r], target_idx[r]); -1 for a row_type
+    outside [0, n_types).  Membership of the target is the caller's: the kernel does not check it.  Returns int64 [R]."""
+    q = q.contiguous()
+    rows, dim = q.shape
+    target_rows = target_rows.contiguous()
+    target_idx = target_idx.contiguous()
+    if tuple(target_rows.shape) != (rows, dim):
+        raise ValueError(f"rank_by_type: target_rows {tuple(target_rows.shape)} != queries {(rows, dim)}")
+    if tuple(target_idx.shape) != (rows,):
+        raise ValueError(f"rank_by_type: target_idx {tuple(target_idx.shape)} != ({rows},)")
+    if row_type is not None and tuple(row_type.shape) != (rows,):
+        raise ValueError(f"rank_by_type: row_type {tuple(row_type.shape)} != ({rows},)")
+    out = torch.empty(rows, dtype=I64, device=q.device)
+    if rows == 0:
+        return out
+    if splits is None:
+        # as topk_by_type for k <= 32
+        n_cat = members.numel() if members is not None else catalog.shape[0]
+        distinct = n_types * (1.0 - math.exp(-rows / max(n_types, 1)))
+        splits = _auto_splits(int(distinct + rows / TOPK_GROUP_ROWS) + 1, n_cat / max(n_types, 1))
+    ws = _lib.workspace(_lib.LIB.pc_rank_by_type_workspace_bytes(rows), q.device)
+    call("pc_rank_by_type", dev(q, F32, "q"), rows, dim, dev(catalog, F32, "catalog"), dev(members, I32, "members"),
+         dev(type_offsets, I64, "type_offsets"), int(n_types), dev(row_type, I32, "row_type"),
+         dev(target_rows, F32, "target_rows"), dev(target_idx, I64, "target_idx"), splits, int(index_base),
+         dev(out, I64, "out_rank"), dev(ws, torch.uint8, "ws"), ws.numel(), stream())
+    return out
+
+
 def score_topk_dense(q: torch.Tensor, catalog: torch.Tensor, k: int, type_id: Optional[torch.Tensor] = None,
                      row_type: Optional[torch.Tensor] = None, index_base: int = 0, max_norm: Optional[float] = None,
                      units: Optional[int] = None):

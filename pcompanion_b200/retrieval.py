@@ -6,12 +6,15 @@
   for every (projected embedding, complementary type) row, rank the products of that type by
   dot product and return the top-k.  The catalog is kept with a type-sorted permutation
   (``BehaviorProductGraph.type_members``), so a row touches only its type's run of products.
+  ``CatalogIndex.rank`` gives the exact position of a target product in that ranking, and
+  ``Metrics.rank_metrics`` turns such ranks into full-catalog hit@k / NDCG@k / MRR.
 * ``ShardedCatalog`` shards the catalog rows over the ranks of a process group; each rank ranks
-  its shard and the per-shard lists are all-gathered and merged (ties -> lowest global index).
+  its shard and the per-shard lists are all-gathered and merged (ties -> lowest global index);
+  per-shard target ranks are added.
 """
 from __future__ import annotations
 
-from typing import Dict, Optional, Tuple
+from typing import Dict, Optional, Sequence, Tuple
 
 import torch
 
@@ -36,6 +39,28 @@ class Metrics:
         _, top_k = ops.topk_rows(predictions.float(), k)
         hits = torch.any(top_k == ground_truth.unsqueeze(1), dim=1)
         return hits.float().mean().item()
+
+    @staticmethod
+    def rank_metrics(ranks: torch.Tensor, ks: Sequence[int] = (1, 3, 10, 50, 100)) -> Dict[str, float]:
+        """Full-catalog retrieval metrics from target ranks (``CatalogIndex.rank``: 0-based, -1 = the target can never
+        be listed), one relevant product per row; every mean is over all rows and a -1 counts as a miss.
+        hit@k = mean(0 <= rank < k), ndcg@k = mean(1 / log2(rank + 2) if 0 <= rank < k else 0),
+        mrr = mean(1 / (rank + 1), 0 for -1), num_rows.  Any k >= 1."""
+        r = ranks.reshape(-1).to(torch.float64)
+        n = r.numel()
+        found = r >= 0
+        out: Dict[str, float] = {}
+        for k in ks:
+            if k < 1:
+                raise ValueError(f"rank_metrics: k={k} must be >= 1")
+            hit = found & (r < k)
+            out[f"hit@{k}"] = hit.double().mean().item() if n else 0.0
+            gain = torch.where(hit, 1.0 / torch.log2(r + 2.0), torch.zeros_like(r))
+            out[f"ndcg@{k}"] = gain.mean().item() if n else 0.0
+        rr = torch.where(found, 1.0 / (r + 1.0), torch.zeros_like(r))
+        out["mrr"] = rr.mean().item() if n else 0.0
+        out["num_rows"] = n
+        return out
 
     @staticmethod
     def type_diversity(predicted_types: torch.Tensor) -> float:
@@ -129,6 +154,53 @@ class CatalogIndex:
             s[bad], i[bad] = fs, fi
         return s, i
 
+    def _owned_targets(self, queries: torch.Tensor, targets: torch.Tensor, row_type: Optional[torch.Tensor]):
+        """(row types int32 or None, member bool [R], target rows fp32 [R, D]) for global target indices: member[r] when
+        this catalog holds targets[r] and, with row types, the target has row r's type.  Rows that are not members get
+        catalog row 0 as a stand-in (an out-of-range index is never gathered)."""
+        rows = queries.shape[0]
+        if tuple(targets.shape) != (rows,):
+            raise ValueError(f"CatalogIndex.rank: targets {tuple(targets.shape)} != ({rows},)")
+        if row_type is not None and self.offsets is None:
+            raise ValueError("CatalogIndex.rank: the catalog was built without type ids")
+        local = targets.to(queries.device, torch.int64) - self.index_base
+        member = (local >= 0) & (local < self.num_products)
+        safe = torch.where(member, local, torch.zeros_like(local))
+        rt = None
+        if row_type is not None:
+            rt = row_type.to(queries.device, torch.int32).reshape(-1).contiguous()
+            if self.num_products:
+                member &= self.type_id[safe] == rt
+        if self.num_products == 0:
+            return rt, member, torch.zeros(rows, queries.shape[1], dtype=torch.float32, device=queries.device)
+        return rt, member, ops.gather_rows(self.catalog, safe)
+
+    def _rank_counts(self, queries: torch.Tensor, target_rows: torch.Tensor, targets: torch.Tensor,
+                     row_type: Optional[torch.Tensor], splits: Optional[int] = None) -> torch.Tensor:
+        """Products of this catalog that rank before each target (pc_rank_by_type; -1 for a row type out of range)."""
+        targets = targets.to(queries.device, torch.int64).contiguous()
+        if self.num_products == 0:
+            return torch.zeros(queries.shape[0], dtype=torch.int64, device=queries.device)
+        if row_type is None:
+            if self._all is None:
+                self._all = torch.tensor([0, self.num_products], dtype=torch.int64, device=queries.device)
+            return ops.rank_by_type(queries, self.catalog, self._all, 1, None, target_rows, targets, None, self.index_base,
+                                    splits)
+        return ops.rank_by_type(queries, self.catalog, self.offsets, self.num_types, row_type, target_rows, targets,
+                                self.members, self.index_base, splits)
+
+    def rank(self, queries: torch.Tensor, targets: torch.Tensor, row_type: Optional[torch.Tensor] = None,
+             splits: Optional[int] = None) -> torch.Tensor:
+        """Exact rank of the product targets[r] (int64 global index) in row r's ranking: the number of products of the
+        row's type (all products when row_type is None) that rank strictly before it, by score descending, then lower
+        index.  -1 when the target can never be listed for the row: it is not in the catalog, or row_type[r] is not its
+        type.  For every k, 0 <= rank < k exactly when ``topk(queries, k, row_type)`` lists the target, and it is then at
+        position rank.  Returns int64 [R]."""
+        queries = queries.contiguous().float()
+        rt, member, target_rows = self._owned_targets(queries, targets, row_type)
+        counts = self._rank_counts(queries, target_rows, targets, rt, splits)
+        return torch.where(member, counts, torch.full_like(counts, -1))
+
     def recommend(self, projected_embeddings: torch.Tensor, complementary_types: torch.Tensor, k: int = 10):
         """The loop of inference.py:93-113 for a whole batch: projected [B, Kt, D], types [B, Kt] ->
         (scores [B, Kt, k], product indices [B, Kt, k]), 1 <= k <= ops.TOPK_MAX_K; a type with fewer than k products
@@ -141,7 +213,8 @@ class CatalogIndex:
 class ShardedCatalog:
     """Catalog rows sharded contiguously over a process group (SURVEY 8e): rank g owns rows
     [bounds[g], bounds[g+1]); queries are replicated; per-shard top-k lists are all-gathered and
-    merged.  Works with NCCL (CUDA tensors) and gloo; the only collective is one [R, 2k] all-gather."""
+    merged.  Works with NCCL (CUDA tensors) and gloo; the only collective of topk is one [R, 2k] all-gather (rank: two
+    all-reduces, [R, D + 1] fp32 and [R] int64)."""
 
     def __init__(self, local_catalog: torch.Tensor, local_type_id: Optional[torch.Tensor], index_base: int,
                  num_types: Optional[int] = None, group=None):
@@ -161,3 +234,23 @@ class ShardedCatalog:
         cat_s = gathered[:, :, :k].permute(1, 0, 2).reshape(s.shape[0], world * k)
         cat_i = gathered[:, :, k:].permute(1, 0, 2).reshape(s.shape[0], world * k).contiguous().view(torch.int64)
         return ops.topk_merge(cat_s, cat_i, k)
+
+    def rank(self, queries: torch.Tensor, targets: torch.Tensor, row_type: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """CatalogIndex.rank over the whole sharded catalog (queries, targets and row types replicated on every rank);
+        equal to the rank on the unsharded catalog.  The shard that owns a target supplies its row and membership (one
+        all-reduce: the other shards add zeros, which change no bit of the row), every shard counts its own products that
+        rank before it, and one all-reduce adds the counts."""
+        import torch.distributed as dist
+        world = dist.get_world_size(self.group) if dist.is_initialized() else 1
+        if world == 1:
+            return self.local.rank(queries, targets, row_type)
+        queries = queries.contiguous().float()
+        rt, member, target_rows = self.local._owned_targets(queries, targets, row_type)
+        packed = torch.cat([torch.where(member[:, None], target_rows, torch.zeros_like(target_rows)),
+                            member[:, None].float()], dim=1).contiguous()
+        dist.all_reduce(packed, op=dist.ReduceOp.SUM, group=self.group)
+        member = packed[:, -1] > 0
+        counts = self.local._rank_counts(queries, packed[:, :-1].contiguous(), targets, rt)
+        counts = counts.clamp_min(0)               # a row type past this shard's type count: none of its products
+        dist.all_reduce(counts, op=dist.ReduceOp.SUM, group=self.group)
+        return torch.where(member, counts, torch.full_like(counts, -1))
