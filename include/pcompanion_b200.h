@@ -253,6 +253,35 @@ int pc_rank_by_type(const float* q, int64_t rows, int dim, const float* catalog,
                     const int64_t* type_offsets, int n_types, const int32_t* row_type, const float* target_rows,
                     const int64_t* target_idx, int splits, int64_t index_base, int64_t* out_rank, void* workspace,
                     size_t workspace_bytes, pc_stream_t stream);
+/* Exclusion lists: row r ignores the products of a list E_r.  Lists hold GLOBAL product indices (int64) in CSR form,
+ * excl_offsets [n_lists + 1] and excl_idx [excl_offsets[n_lists]], ascending within each list, duplicates allowed.
+ * row_list [rows] (int32) maps score row r to its list; a value outside [0, n_lists) means no exclusions; row_list NULL:
+ * row r uses list r.  Entries outside this catalog (shard) or of another type have no effect, so one set of lists
+ * serves every shard unchanged.  n_lists == 0: no row has exclusions (the list pointers may be NULL).
+ *
+ * pc_topk_by_type_excluding: the exact top-k of row r's run with the products of E_r removed.  Arguments,
+ * workspace (pc_topk_by_type_workspace_bytes), ranking rule, score bits, (-inf, -1) padding and reproducibility are
+ * those of pc_topk_by_type; with every list empty the output equals pc_topk_by_type bit for bit.  A product is
+ * looked up in E_r (binary search) only after it ranks before the current k-th entry of its row. */
+int pc_topk_by_type_excluding(const float* q, int64_t rows, int dim, const float* catalog, const int32_t* members,
+                              const int64_t* type_offsets, int n_types, const int32_t* row_type, int k, int splits,
+                              int64_t index_base, const int64_t* excl_offsets, const int64_t* excl_idx, int64_t n_lists,
+                              const int32_t* row_list, double* out_scores, int64_t* out_idx, void* workspace,
+                              size_t workspace_bytes, pc_stream_t stream);
+/* Filtered rank: run after pc_rank_by_type on the same stream with the same q, catalog, target_rows, target_idx,
+ * row_type and index_base.  For every row with inout_rank[r] >= 0 it subtracts the number of DISTINCT entries e of E_r
+ * that are local (index_base <= e < index_base + n_products), of row r's type (type_id [n_products] int32 is the
+ * catalog's local type of each row; any local product when row_type is NULL, i.e. the run is the whole catalog) and
+ * whose (score(q[r], e), e) ranks strictly before (score(q[r], target_rows[r]), target_idx[r]).  Both scores use the
+ * streaming pass's arithmetic in its order, so they are the bits pc_rank_by_type compared: the result is the number of
+ * products of the run that are not in E_r and rank before the target, and a target listed in E_r never removes
+ * itself.  For every k, 0 <= rank < k exactly when pc_topk_by_type_excluding with E_r - {target} lists the target, at
+ * position rank.  One warp per row; rows -1 stay -1. */
+int pc_rank_remove_excluded(const float* q, int64_t rows, int dim, const float* catalog, int64_t n_products,
+                            const int32_t* type_id, const int32_t* row_type, const float* target_rows,
+                            const int64_t* target_idx, int64_t index_base, const int64_t* excl_offsets,
+                            const int64_t* excl_idx, int64_t n_lists, const int32_t* row_list, int64_t* inout_rank,
+                            pc_stream_t stream);
 /* Dense whole-catalog variant on the tensor cores (north_star part 4): scores = Q . C^T as a TF32 tcgen05
  * GEMM (never materialised; approximate scores only select candidates), per-type mask (type_id[p] == row_type[r]; row_type NULL or < 0 = no mask) and a
  * per-row candidate list fused into the epilogue, then exact float64 re-scoring + ranking of the candidates.

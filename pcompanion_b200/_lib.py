@@ -65,6 +65,9 @@ PROTOTYPES = {
     "pc_topk_by_type": (c_int, [P, c_int64, c_int, P, P, P, c_int, P, c_int, c_int, c_int64, P, P, P, c_size_t, P]),
     "pc_rank_by_type_workspace_bytes": (c_size_t, [c_int64]),
     "pc_rank_by_type": (c_int, [P, c_int64, c_int, P, P, P, c_int, P, P, P, c_int, c_int64, P, P, c_size_t, P]),
+    "pc_topk_by_type_excluding": (c_int, [P, c_int64, c_int, P, P, P, c_int, P, c_int, c_int, c_int64, P, P, c_int64, P, P, P,
+                                          P, c_size_t, P]),
+    "pc_rank_remove_excluded": (c_int, [P, c_int64, c_int, P, c_int64, P, P, P, P, c_int64, P, P, c_int64, P, P, P]),
     "pc_score_topk_workspace_bytes": (c_size_t, [c_int64, c_int]),
     "pc_score_topk_dense": (c_int, [P, c_int64, c_int, P, c_int64, P, P, c_int, c_int, c_int64, c_float, P, P, P, P, c_size_t, P]),
     "pc_topk_rows_workspace_bytes": (c_size_t, [c_int64, c_int, c_int]),

@@ -56,6 +56,40 @@ __device__ __forceinline__ void warp_topk_insert(Cand& mine, int k, double s, in
   }
 }
 
+// Exclusion lists (pc_topk_by_type_excluding, pc_rank_remove_excluded): CSR lists of global product indices, ascending
+// within each list (duplicates allowed).  Score row r uses list row_list[r] (list r when row_list is NULL); a list id
+// outside [0, n_lists) means no exclusions.
+struct Excl {
+  const int64_t* offsets;
+  const int64_t* idx;
+  int64_t n_lists;
+  const int32_t* row_list;
+};
+
+// [lo, hi) of score row `row`'s list
+__device__ __forceinline__ void excl_bounds(const Excl ex, int64_t row, int64_t& lo, int64_t& hi) {
+  const int64_t l = ex.row_list ? int64_t(ex.row_list[row]) : row;
+  lo = hi = 0;
+  if (l >= 0 && l < ex.n_lists) {
+    lo = ex.offsets[l];
+    hi = ex.offsets[l + 1];
+  }
+}
+
+// g is among idx[lo .. hi) (ascending): binary search for the last entry <= g, on a pointer and a 32-bit count so that
+// it fits the k <= 32 kernel's registers (a list holds < 2^31 entries)
+__device__ __forceinline__ bool excl_listed(const int64_t* __restrict__ idx, int64_t lo, int64_t hi, int64_t g) {
+  if (lo >= hi) return false;
+  const int64_t* base = idx + lo;
+  int n = int(hi - lo);
+  while (n > 1) {
+    const int half = n >> 1;
+    if (base[half] <= g) base += half;
+    n -= half;
+  }
+  return *base == g;
+}
+
 constexpr int RB = 8;            // score rows per group
 constexpr int DCH = 16;          // dims per staged chunk
 constexpr int TILE_LD = 20;      // floats per staged product chunk (16 + 4 pad: conflict-free LDS.128 across lanes)
@@ -136,18 +170,33 @@ __device__ __forceinline__ void score_pass(double (&acc)[PP][R], float* tile, in
 // members[seg_begin[g] .. seg_end[g]).  A lane owns PP products of a BATCH-product pass; 32-dim chunks are staged
 // through shared memory with cp.async (double-buffered, coalesced), then every lane advances PP x RB independent
 // sequential fp64 dot products (the chains interleave, which is what keeps the fp64 pipe busy).
+// EXCL: a product whose global index is in its row's exclusion list never enters the row's list.  It is tested only
+// after it ranks before the warp's current k-th entry, so the list is searched for few products.  The rows' list
+// bounds sit in shared memory after the tile area (the k <= 32 kernel is capped at 128 registers).
+template <bool EXCL>
 __device__ __forceinline__ void topk_group_body(const float* __restrict__ Q, int dim, const float* __restrict__ catalog,
                                                 const int32_t* __restrict__ members, const int32_t* __restrict__ row_ids,
                                                 int r_beg, int n_rows, int64_t beg, int64_t end, int k, int splits, int split,
-                                                int64_t index_base, double* __restrict__ part_s, int64_t* __restrict__ part_i) {
+                                                int64_t index_base, double* __restrict__ part_s, int64_t* __restrict__ part_i,
+                                                const Excl ex) {
   extern __shared__ double smem_d[];
   double* q_s = smem_d;                                                      // [RB][dim], rows >= n_rows are zero
   float* tiles = reinterpret_cast<float*>(q_s + RB * dim);                   // [TK_WARPS][2][BATCH][TILE_LD]
   Cand* lists = reinterpret_cast<Cand*>(tiles);                              // [TK_WARPS][RB][32], reuses the tile area after the scan
+  int64_t* ex_lo = reinterpret_cast<int64_t*>(tiles + TK_WARPS * 2 * TILE_FLOATS);  // EXCL: [RB] list begin, then [RB] end
+  static_assert(TK_WARPS * 2 * TILE_FLOATS * sizeof(float) >= TK_WARPS * RB * 32 * sizeof(Cand), "lists fit the tile area");
   const int lane = lane_id(), w = warp_id();
   for (int i = threadIdx.x; i < RB * dim; i += blockDim.x) {
     const int r = i / dim, d = i - r * dim;
     q_s[i] = r < n_rows ? double(Q[int64_t(row_ids[r_beg + r]) * dim + d]) : 0.0;
+  }
+  if constexpr (EXCL) {
+    if (threadIdx.x < RB) {
+      int64_t lo = 0, hi = 0;
+      if (int(threadIdx.x) < n_rows) excl_bounds(ex, row_ids[r_beg + threadIdx.x], lo, hi);
+      ex_lo[threadIdx.x] = lo;
+      ex_lo[RB + threadIdx.x] = hi;
+    }
   }
   __syncthreads();
   const int64_t len = end > beg ? end - beg : 0;
@@ -217,7 +266,9 @@ __device__ __forceinline__ void topk_group_body(const float* __restrict__ Q, int
         if (r < n_rows) {
           const double thr_s = shfl_d(mine[r].s, k - 1);
           const int64_t thr_i = shfl_i64(mine[r].i, k - 1);
-          uint32_t cand = __ballot_sync(FULL, gidx >= 0 && ranks_before(acc[pp][r], gidx, thr_s, thr_i));
+          bool take = gidx >= 0 && ranks_before(acc[pp][r], gidx, thr_s, thr_i);
+          if constexpr (EXCL) take = take && !excl_listed(ex.idx, ex_lo[r], ex_lo[RB + r], gidx);
+          uint32_t cand = __ballot_sync(FULL, take);
           while (cand) {
             const int src = __ffs(cand) - 1;
             cand &= cand - 1;
@@ -261,8 +312,8 @@ topk_groups_kernel(const float* __restrict__ Q, int dim, const float* __restrict
                    double* __restrict__ part_s, int64_t* __restrict__ part_i) {
   const int g = blockIdx.y;
   const int r_beg = grp_begin[g];
-  topk_group_body(Q, dim, catalog, members, row_ids, r_beg, grp_begin[g + 1] - r_beg, seg_begin[g], seg_end[g], k, splits,
-                  int(blockIdx.x), index_base, part_s, part_i);
+  topk_group_body<false>(Q, dim, catalog, members, row_ids, r_beg, grp_begin[g + 1] - r_beg, seg_begin[g], seg_end[g], k,
+                         splits, int(blockIdx.x), index_base, part_s, part_i, Excl{});
 }
 
 // ---- device-side grouping (pc_topk_by_type): no host read-back anywhere between the query upload and the result.
@@ -312,8 +363,24 @@ topk_planned_kernel(const float* __restrict__ Q, int dim, const float* __restric
   if (n_rows == 0) return;                      // uniform over the CTA
   const int64_t t = int64_t(keys[p] >> 32);
   const int64_t beg = t < n_types ? type_offsets[t] : 0, end = t < n_types ? type_offsets[t + 1] : 0;
-  topk_group_body(Q, dim, catalog, members, row_ids, int(p), n_rows, beg, end, k, splits, int(blockIdx.x), index_base,
-                  part_s, part_i);
+  topk_group_body<false>(Q, dim, catalog, members, row_ids, int(p), n_rows, beg, end, k, splits, int(blockIdx.x), index_base,
+                         part_s, part_i, Excl{});
+}
+
+// topk_planned_kernel with exclusion lists (pc_topk_by_type_excluding, k <= 32)
+__global__ void __launch_bounds__(TK_WARPS * 32, 2)
+topk_planned_excl_kernel(const float* __restrict__ Q, int dim, const float* __restrict__ catalog,
+                         const int32_t* __restrict__ members, const int32_t* __restrict__ row_ids,
+                         const int32_t* __restrict__ grp_rows, const uint64_t* __restrict__ keys,
+                         const int64_t* __restrict__ type_offsets, int n_types, int64_t p0, int k, int splits,
+                         int64_t index_base, double* __restrict__ part_s, int64_t* __restrict__ part_i, const Excl ex) {
+  const int64_t p = p0 + blockIdx.y;
+  const int n_rows = grp_rows[p];
+  if (n_rows == 0) return;                      // uniform over the CTA
+  const int64_t t = int64_t(keys[p] >> 32);
+  const int64_t beg = t < n_types ? type_offsets[t] : 0, end = t < n_types ? type_offsets[t + 1] : 0;
+  topk_group_body<true>(Q, dim, catalog, members, row_ids, int(p), n_rows, beg, end, k, splits, int(blockIdx.x), index_base,
+                        part_s, part_i, ex);
 }
 
 // row-wise top-k of a materialised fp32 matrix: grid = (splits, rows)
@@ -462,13 +529,14 @@ __device__ void compact_rows(double* bs, IdxT* bi, int cap, int* cnt, double* th
 }
 
 // Large-k counterpart of topk_group_body for R score rows (R * cap buffer entries fit beside the staged tiles).  The
-// scoring is score_pass, so the scores are the same bits as the k <= 32 kernel's.
-template <int R>
+// scoring is score_pass, so the scores are the same bits as the k <= 32 kernel's.  EXCL: as topk_group_body, the
+// exclusion test follows the threshold test; the list bounds follow `cnt` in shared memory.
+template <int R, bool EXCL>
 __device__ __forceinline__ void topk_group_large_body(const float* __restrict__ Q, int dim, const float* __restrict__ catalog,
                                                       const int32_t* __restrict__ members, const int32_t* __restrict__ row_ids,
                                                       int r_beg, int n_rows, int64_t beg, int64_t end, int k, int cap, int splits,
                                                       int split, int64_t index_base, double* __restrict__ part_s,
-                                                      int64_t* __restrict__ part_i) {
+                                                      int64_t* __restrict__ part_i, const Excl ex) {
   extern __shared__ double smem_d[];
   double* q_s = smem_d;                                                      // [R][dim], rows >= n_rows are zero
   float* tiles = reinterpret_cast<float*>(q_s + R * dim);                    // [TK_WARPS][2][BATCH][TILE_LD]
@@ -477,6 +545,7 @@ __device__ __forceinline__ void topk_group_large_body(const float* __restrict__ 
   int32_t* bi = reinterpret_cast<int32_t*>(thr_s + R);                       // [R][cap] catalog row ids
   int32_t* thr_i = bi + R * cap;                                             // [R]
   int* cnt = thr_i + R;                                                      // [R]
+  int64_t* ex_lo = reinterpret_cast<int64_t*>((reinterpret_cast<uintptr_t>(cnt + R) + 7) & ~uintptr_t(7));  // EXCL: [R] begin, [R] end
   const int lane = lane_id(), w = warp_id();
   for (int i = threadIdx.x; i < R * dim; i += blockDim.x) {
     const int r = i / dim, d = i - r * dim;
@@ -486,6 +555,12 @@ __device__ __forceinline__ void topk_group_large_body(const float* __restrict__ 
     cnt[threadIdx.x] = 0;
     thr_s[threadIdx.x] = -INFINITY;
     thr_i[threadIdx.x] = -1;
+    if constexpr (EXCL) {
+      int64_t lo = 0, hi = 0;
+      if (int(threadIdx.x) < n_rows) excl_bounds(ex, row_ids[r_beg + threadIdx.x], lo, hi);
+      ex_lo[threadIdx.x] = lo;
+      ex_lo[R + threadIdx.x] = hi;
+    }
   }
   __syncthreads();
   const int64_t len = end > beg ? end - beg : 0;
@@ -513,7 +588,8 @@ __device__ __forceinline__ void topk_group_large_body(const float* __restrict__ 
 #pragma unroll
       for (int r = 0; r < R; ++r) {
         if (r < n_rows) {
-          const bool take = cur[pp] >= 0 && ranks_before(acc[pp][r], cur[pp], thr_s[r], thr_i[r]);
+          bool take = cur[pp] >= 0 && ranks_before(acc[pp][r], cur[pp], thr_s[r], thr_i[r]);
+          if constexpr (EXCL) take = take && !excl_listed(ex.idx, ex_lo[r], ex_lo[R + r], int64_t(cur[pp]) + index_base);
           append_candidate<int32_t>(take, acc[pp][r], cur[pp], bs + r * cap, bi + r * cap, cnt + r);
         }
       }
@@ -551,8 +627,8 @@ topk_groups_large_kernel(const float* __restrict__ Q, int dim, const float* __re
   const int r_beg = grp_begin[g] + int(blockIdx.z) * R;
   const int n_rows = min(grp_begin[g + 1] - r_beg, R);
   if (n_rows <= 0) return;                      // uniform over the CTA
-  topk_group_large_body<R>(Q, dim, catalog, members, row_ids, r_beg, n_rows, seg_begin[g], seg_end[g], k, cap, splits,
-                           int(blockIdx.x), index_base, part_s, part_i);
+  topk_group_large_body<R, false>(Q, dim, catalog, members, row_ids, r_beg, n_rows, seg_begin[g], seg_end[g], k, cap,
+                                  splits, int(blockIdx.x), index_base, part_s, part_i, Excl{});
 }
 
 // pc_topk_by_type's large-k ranking kernel: the plan formed groups of R rows, so one CTA ranks a whole group
@@ -568,8 +644,25 @@ topk_planned_large_kernel(const float* __restrict__ Q, int dim, const float* __r
   if (n_rows == 0) return;                      // uniform over the CTA
   const int64_t t = int64_t(keys[p] >> 32);
   const int64_t beg = t < n_types ? type_offsets[t] : 0, end = t < n_types ? type_offsets[t + 1] : 0;
-  topk_group_large_body<R>(Q, dim, catalog, members, row_ids, int(p), n_rows, beg, end, k, cap, splits, int(blockIdx.x),
-                           index_base, part_s, part_i);
+  topk_group_large_body<R, false>(Q, dim, catalog, members, row_ids, int(p), n_rows, beg, end, k, cap, splits,
+                                  int(blockIdx.x), index_base, part_s, part_i, Excl{});
+}
+
+// topk_planned_large_kernel with exclusion lists (pc_topk_by_type_excluding, k > 32)
+template <int R>
+__global__ void __launch_bounds__(LK_THREADS, 1)
+topk_planned_large_excl_kernel(const float* __restrict__ Q, int dim, const float* __restrict__ catalog,
+                               const int32_t* __restrict__ members, const int32_t* __restrict__ row_ids,
+                               const int32_t* __restrict__ grp_rows, const uint64_t* __restrict__ keys,
+                               const int64_t* __restrict__ type_offsets, int n_types, int64_t p0, int k, int cap, int splits,
+                               int64_t index_base, double* __restrict__ part_s, int64_t* __restrict__ part_i, const Excl ex) {
+  const int64_t p = p0 + blockIdx.y;
+  const int n_rows = grp_rows[p];
+  if (n_rows == 0) return;                      // uniform over the CTA
+  const int64_t t = int64_t(keys[p] >> 32);
+  const int64_t beg = t < n_types ? type_offsets[t] : 0, end = t < n_types ? type_offsets[t + 1] : 0;
+  topk_group_large_body<R, true>(Q, dim, catalog, members, row_ids, int(p), n_rows, beg, end, k, cap, splits,
+                                 int(blockIdx.x), index_base, part_s, part_i, ex);
 }
 
 // Large-k selection over one row's stream of n (score, index) items, LK_STREAM_PASS items per pass; index < 0 is
@@ -672,19 +765,27 @@ int launch_groups_large(const float* q, int dim, const float* catalog, const int
   return PC_OK;
 }
 
+// ex == nullptr: no exclusion lists (topk_planned_large_kernel)
 template <int R>
 int launch_by_type_large(const float* q, int64_t rows, int dim, const float* catalog, const int32_t* members,
                          const int64_t* type_offsets, int n_types, const uint64_t* keys, int32_t* row_ids, int32_t* grp_rows,
-                         int k, int cap, int splits, int64_t index_base, double* ps, int64_t* pi, cudaStream_t st) {
+                         int k, int cap, int splits, int64_t index_base, double* ps, int64_t* pi, const Excl* ex,
+                         cudaStream_t st) {
   topk_plan_kernel<R><<<unsigned(ceil_div(rows, 256)), 256, 0, st>>>(keys, rows, row_ids, grp_rows);
   PC_LAUNCH_CHECK();
-  const size_t smem = group_large_smem(R, cap, dim);
-  PC_CUDA(cudaFuncSetAttribute(topk_planned_large_kernel<R>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+  const size_t smem = group_large_smem(R, cap, dim) + (ex ? 8 + 2 * R * sizeof(int64_t) : 0);   // + aligned list bounds
+  if (ex) PC_CUDA(cudaFuncSetAttribute(topk_planned_large_excl_kernel<R>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+  else PC_CUDA(cudaFuncSetAttribute(topk_planned_large_kernel<R>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
   for (int64_t p0 = 0; p0 < rows; p0 += 65535) {   // gridDim.y limit
     const int64_t np = rows - p0 < 65535 ? rows - p0 : 65535;
     dim3 grid{unsigned(splits), unsigned(np), 1u};
-    topk_planned_large_kernel<R><<<grid, LK_THREADS, smem, st>>>(q, dim, catalog, members, row_ids, grp_rows, keys,
-                                                                type_offsets, n_types, p0, k, cap, splits, index_base, ps, pi);
+    if (ex)
+      topk_planned_large_excl_kernel<R><<<grid, LK_THREADS, smem, st>>>(q, dim, catalog, members, row_ids, grp_rows, keys,
+                                                                       type_offsets, n_types, p0, k, cap, splits, index_base,
+                                                                       ps, pi, *ex);
+    else
+      topk_planned_large_kernel<R><<<grid, LK_THREADS, smem, st>>>(q, dim, catalog, members, row_ids, grp_rows, keys,
+                                                                  type_offsets, n_types, p0, k, cap, splits, index_base, ps, pi);
     PC_LAUNCH_CHECK();
   }
   return PC_OK;
@@ -704,13 +805,13 @@ int groups_large(const float* q, int dim, const float* catalog, const int32_t* m
 
 int by_type_large(const float* q, int64_t rows, int dim, const float* catalog, const int32_t* members,
                   const int64_t* type_offsets, int n_types, const uint64_t* keys, int32_t* row_ids, int32_t* grp_rows, int k,
-                  int splits, int64_t index_base, double* ps, int64_t* pi, cudaStream_t st) {
+                  int splits, int64_t index_base, double* ps, int64_t* pi, const Excl* ex, cudaStream_t st) {
   const int cap = large_cap(k, LK_GROUP_PASS);
   switch (group_large_rows(cap, dim)) {
-    case 8: return launch_by_type_large<8>(q, rows, dim, catalog, members, type_offsets, n_types, keys, row_ids, grp_rows, k, cap, splits, index_base, ps, pi, st);
-    case 4: return launch_by_type_large<4>(q, rows, dim, catalog, members, type_offsets, n_types, keys, row_ids, grp_rows, k, cap, splits, index_base, ps, pi, st);
-    case 2: return launch_by_type_large<2>(q, rows, dim, catalog, members, type_offsets, n_types, keys, row_ids, grp_rows, k, cap, splits, index_base, ps, pi, st);
-    default: return launch_by_type_large<1>(q, rows, dim, catalog, members, type_offsets, n_types, keys, row_ids, grp_rows, k, cap, splits, index_base, ps, pi, st);
+    case 8: return launch_by_type_large<8>(q, rows, dim, catalog, members, type_offsets, n_types, keys, row_ids, grp_rows, k, cap, splits, index_base, ps, pi, ex, st);
+    case 4: return launch_by_type_large<4>(q, rows, dim, catalog, members, type_offsets, n_types, keys, row_ids, grp_rows, k, cap, splits, index_base, ps, pi, ex, st);
+    case 2: return launch_by_type_large<2>(q, rows, dim, catalog, members, type_offsets, n_types, keys, row_ids, grp_rows, k, cap, splits, index_base, ps, pi, ex, st);
+    default: return launch_by_type_large<1>(q, rows, dim, catalog, members, type_offsets, n_types, keys, row_ids, grp_rows, k, cap, splits, index_base, ps, pi, ex, st);
   }
 }
 
@@ -807,6 +908,53 @@ rank_planned_kernel(const float* __restrict__ Q, int dim, const float* __restric
   if (threadIdx.x < n_rows && cnt_s[threadIdx.x]) atomicAdd(out_rank + row_ids[p + threadIdx.x], cnt_s[threadIdx.x]);
 }
 
+// s = sum_d q[d] * c[d] with the streaming pass's arithmetic in its order: fma(double(q[d]), double(c[d]), s), d ascending
+// from 0 (dim % 16 == 0, rows 16-byte aligned)
+__device__ __forceinline__ double dot_stream_order(const float* __restrict__ q, const float* __restrict__ c, int dim) {
+  double s = 0.0;
+  for (int d = 0; d < dim; d += 4) {
+    const float4 a = __ldg(reinterpret_cast<const float4*>(q + d)), b = __ldg(reinterpret_cast<const float4*>(c + d));
+    s = fma(double(a.x), double(b.x), s);
+    s = fma(double(a.y), double(b.y), s);
+    s = fma(double(a.z), double(b.z), s);
+    s = fma(double(a.w), double(b.w), s);
+  }
+  return s;
+}
+
+// pc_rank_remove_excluded: one warp per score row, lanes stride the row's list.  An entry is subtracted when it is
+// distinct (not equal to its predecessor), local, of the row's type and ranks strictly before the target.  Both scores
+// have the streaming pass's bits, so every subtracted entry is one that pc_rank_by_type counted, and a target listed
+// in its own list never is.
+__global__ void __launch_bounds__(256, 4)
+rank_remove_excluded_kernel(const float* __restrict__ Q, int64_t rows, int dim, const float* __restrict__ catalog,
+                            int64_t n_products, const int32_t* __restrict__ type_id, const int32_t* __restrict__ row_type,
+                            const float* __restrict__ target_rows, const int64_t* __restrict__ target_idx,
+                            int64_t index_base, const Excl ex, int64_t* __restrict__ inout_rank) {
+  const int64_t r = int64_t(blockIdx.x) * 8 + warp_id();
+  if (r >= rows) return;                        // uniform over the warp, as every early return below
+  const int64_t rank = inout_rank[r];
+  if (rank < 0) return;
+  int64_t lo, hi;
+  excl_bounds(ex, r, lo, hi);
+  if (lo >= hi) return;
+  const int lane = lane_id();
+  const float* qr = Q + r * dim;
+  const double ts = dot_stream_order(qr, target_rows + r * dim, dim);
+  const int64_t tg = target_idx[r];
+  const int t = row_type ? row_type[r] : 0;
+  unsigned c = 0;
+  for (int64_t j = lo + lane; j < hi; j += 32) {
+    const int64_t e = ex.idx[j];
+    const int64_t loc = e - index_base;
+    if ((j > lo && ex.idx[j - 1] == e) || loc < 0 || loc >= n_products) continue;
+    if (row_type && type_id[loc] != t) continue;
+    c += ranks_before(dot_stream_order(qr, catalog + loc * dim, dim), e, ts, tg) ? 1u : 0u;
+  }
+  c = __reduce_add_sync(FULL, c);
+  if (lane == 0 && c) inout_rank[r] = rank - int64_t(c);
+}
+
 }  // namespace
 }  // namespace pc
 
@@ -865,10 +1013,11 @@ extern "C" size_t pc_topk_by_type_workspace_bytes(int64_t rows, int k, int split
          pc_topk_groups_workspace_bytes(rows, k, splits);
 }
 
-extern "C" int pc_topk_by_type(const float* q, int64_t rows, int dim, const float* catalog, const int32_t* members,
-                               const int64_t* type_offsets, int n_types, const int32_t* row_type, int k, int splits,
-                               int64_t index_base, double* out_scores, int64_t* out_idx, void* workspace,
-                               size_t workspace_bytes, pc_stream_t stream) {
+// pc_topk_by_type (ex == nullptr) and pc_topk_by_type_excluding: the same grouping, splits and merge
+static int topk_by_type_impl(const float* q, int64_t rows, int dim, const float* catalog, const int32_t* members,
+                             const int64_t* type_offsets, int n_types, const int32_t* row_type, int k, int splits,
+                             int64_t index_base, double* out_scores, int64_t* out_idx, void* workspace,
+                             size_t workspace_bytes, const Excl* ex, pc_stream_t stream) {
   PC_REQUIRE(rows >= 0 && rows < (int64_t(1) << 31), PC_ERR_INVALID, "topk_by_type: bad row count");
   if (rows == 0) return PC_OK;
   PC_REQUIRE(q && catalog && type_offsets && out_scores && out_idx && workspace, PC_ERR_INVALID, "topk_by_type: null pointer");
@@ -900,7 +1049,7 @@ extern "C" int pc_topk_by_type(const float* q, int64_t rows, int dim, const floa
   }
   if (k > WARP_K) {
     if (int rc = by_type_large(q, rows, dim, catalog, members, type_offsets, n_types, keys, row_ids, grp_rows, k, splits,
-                               index_base, ps, pi, st))
+                               index_base, ps, pi, ex, st))
       return rc;
   } else {
     topk_plan_kernel<RB><<<tb, 256, 0, st>>>(keys, rows, row_ids, grp_rows);
@@ -908,17 +1057,42 @@ extern "C" int pc_topk_by_type(const float* q, int64_t rows, int dim, const floa
     const size_t smem = size_t(RB) * dim * sizeof(double) +
                         std::max(size_t(TK_WARPS) * 2 * TILE_FLOATS * sizeof(float), size_t(TK_WARPS) * RB * 32 * sizeof(Cand));
     PC_REQUIRE(smem <= 200 * 1024, PC_ERR_UNSUPPORTED, "topk_by_type: shared memory budget exceeded");
-    PC_CUDA(cudaFuncSetAttribute(topk_planned_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    if (ex) PC_CUDA(cudaFuncSetAttribute(topk_planned_excl_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    else PC_CUDA(cudaFuncSetAttribute(topk_planned_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
     for (int64_t p0 = 0; p0 < rows; p0 += 65535) {   // gridDim.y limit
       const int64_t np = rows - p0 < 65535 ? rows - p0 : 65535;
       dim3 grid{unsigned(splits), unsigned(np), 1u};
-      topk_planned_kernel<<<grid, TK_WARPS * 32, smem, st>>>(q, dim, catalog, members, row_ids, grp_rows, keys, type_offsets,
-                                                             n_types, p0, k, splits, index_base, ps, pi);
+      if (ex)   // + the rows' list bounds after the tile area
+        topk_planned_excl_kernel<<<grid, TK_WARPS * 32, smem + 2 * RB * sizeof(int64_t), st>>>(
+            q, dim, catalog, members, row_ids, grp_rows, keys, type_offsets, n_types, p0, k, splits, index_base, ps, pi, *ex);
+      else
+        topk_planned_kernel<<<grid, TK_WARPS * 32, smem, st>>>(q, dim, catalog, members, row_ids, grp_rows, keys, type_offsets,
+                                                               n_types, p0, k, splits, index_base, ps, pi);
       PC_LAUNCH_CHECK();
     }
   }
   if (splits > 1) return pc_topk_merge(ps, pi, rows, splits, k, out_scores, out_idx, stream);
   return PC_OK;
+}
+
+extern "C" int pc_topk_by_type(const float* q, int64_t rows, int dim, const float* catalog, const int32_t* members,
+                               const int64_t* type_offsets, int n_types, const int32_t* row_type, int k, int splits,
+                               int64_t index_base, double* out_scores, int64_t* out_idx, void* workspace,
+                               size_t workspace_bytes, pc_stream_t stream) {
+  return topk_by_type_impl(q, rows, dim, catalog, members, type_offsets, n_types, row_type, k, splits, index_base,
+                           out_scores, out_idx, workspace, workspace_bytes, nullptr, stream);
+}
+
+extern "C" int pc_topk_by_type_excluding(const float* q, int64_t rows, int dim, const float* catalog, const int32_t* members,
+                                         const int64_t* type_offsets, int n_types, const int32_t* row_type, int k, int splits,
+                                         int64_t index_base, const int64_t* excl_offsets, const int64_t* excl_idx,
+                                         int64_t n_lists, const int32_t* row_list, double* out_scores, int64_t* out_idx,
+                                         void* workspace, size_t workspace_bytes, pc_stream_t stream) {
+  PC_REQUIRE(n_lists >= 0, PC_ERR_INVALID, "topk_by_type_excluding: n_lists=%lld < 0", (long long)n_lists);
+  PC_REQUIRE(n_lists == 0 || (excl_offsets && excl_idx), PC_ERR_INVALID, "topk_by_type_excluding: null exclusion lists");
+  const Excl ex{excl_offsets, excl_idx, n_lists, row_list};
+  return topk_by_type_impl(q, rows, dim, catalog, members, type_offsets, n_types, row_type, k, splits, index_base,
+                           out_scores, out_idx, workspace, workspace_bytes, &ex, stream);
 }
 
 extern "C" size_t pc_rank_by_type_workspace_bytes(int64_t rows) {
@@ -966,6 +1140,24 @@ extern "C" int pc_rank_by_type(const float* q, int64_t rows, int dim, const floa
                                                            reinterpret_cast<unsigned long long*>(out_rank));
     PC_LAUNCH_CHECK();
   }
+  return PC_OK;
+}
+
+extern "C" int pc_rank_remove_excluded(const float* q, int64_t rows, int dim, const float* catalog, int64_t n_products,
+                                       const int32_t* type_id, const int32_t* row_type, const float* target_rows,
+                                       const int64_t* target_idx, int64_t index_base, const int64_t* excl_offsets,
+                                       const int64_t* excl_idx, int64_t n_lists, const int32_t* row_list,
+                                       int64_t* inout_rank, pc_stream_t stream) {
+  PC_REQUIRE(rows >= 0 && n_products >= 0 && n_lists >= 0, PC_ERR_INVALID, "rank_remove_excluded: negative size");
+  if (rows == 0 || n_lists == 0 || n_products == 0) return PC_OK;
+  PC_REQUIRE(q && catalog && target_rows && target_idx && excl_offsets && excl_idx && inout_rank, PC_ERR_INVALID,
+             "rank_remove_excluded: null pointer");
+  PC_REQUIRE(!row_type || type_id, PC_ERR_INVALID, "rank_remove_excluded: row_type needs type_id");
+  PC_REQUIRE(dim >= DCH && dim % DCH == 0 && dim <= 1024, PC_ERR_UNSUPPORTED, "rank_remove_excluded: dim=%d must be a multiple of %d (<= 1024)", dim, DCH);
+  const Excl ex{excl_offsets, excl_idx, n_lists, row_list};
+  rank_remove_excluded_kernel<<<unsigned(ceil_div(rows, 8)), 256, 0, as_stream(stream)>>>(
+      q, rows, dim, catalog, n_products, type_id, row_type, target_rows, target_idx, index_base, ex, inout_rank);
+  PC_LAUNCH_CHECK();
   return PC_OK;
 }
 

@@ -827,11 +827,24 @@ def topk_segments(q: torch.Tensor, catalog: torch.Tensor, seg_begin: torch.Tenso
     return out_s, out_i
 
 
+def _exclusion_args(exclude, rows: int, what: str):
+    """(excl_offsets, excl_idx, n_lists, row_list) pointers of a retrieval.Exclusions for `rows` score rows."""
+    if exclude.row_list is not None and tuple(exclude.row_list.shape) != (rows,):
+        raise ValueError(f"{what}: exclusion row_list {tuple(exclude.row_list.shape)} != ({rows},)")
+    idx = exclude.indices
+    if idx.numel() == 0:                        # every list is empty; the kernel still wants a valid pointer
+        idx = torch.zeros(1, dtype=I64, device=idx.device)
+    return (dev(exclude.offsets, I64, "excl_offsets"), dev(idx, I64, "excl_idx"), exclude.num_lists,
+            dev(exclude.row_list, I32, "row_list"))
+
+
 def topk_by_type(q: torch.Tensor, catalog: torch.Tensor, type_offsets: torch.Tensor, n_types: int,
                  row_type: Optional[torch.Tensor], k: int, members: Optional[torch.Tensor] = None, index_base: int = 0,
-                 splits: Optional[int] = None):
+                 splits: Optional[int] = None, exclude=None):
     """Exact top-k of every row over the catalog rows of its type, grouping done on the device (pc_topk_by_type): no
-    host synchronisation between the inputs and the result.  Returns (scores f64 [R,k], idx i64 [R,k])."""
+    host synchronisation between the inputs and the result.  Returns (scores f64 [R,k], idx i64 [R,k]).
+    exclude (retrieval.Exclusions of global indices): row r's list is left out of its ranking
+    (pc_topk_by_type_excluding)."""
     _check_k(k, "topk_by_type")
     q = q.contiguous()
     rows, dim = q.shape
@@ -845,6 +858,12 @@ def topk_by_type(q: torch.Tensor, catalog: torch.Tensor, type_offsets: torch.Ten
         distinct = n_types * (1.0 - math.exp(-rows / max(n_types, 1)))
         splits = _auto_splits(int(distinct + rows / TOPK_GROUP_ROWS) + 1, n_cat / max(n_types, 1), k, rows)
     ws = _lib.workspace(_lib.LIB.pc_topk_by_type_workspace_bytes(rows, k, splits), q.device)
+    if exclude is not None:
+        call("pc_topk_by_type_excluding", dev(q, F32, "q"), rows, dim, dev(catalog, F32, "catalog"),
+             dev(members, I32, "members"), dev(type_offsets, I64, "type_offsets"), int(n_types), dev(row_type, I32, "row_type"),
+             k, splits, int(index_base), *_exclusion_args(exclude, rows, "topk_by_type"), dev(out_s, F64, "out_scores"),
+             dev(out_i, I64, "out_idx"), dev(ws, torch.uint8, "ws"), ws.numel(), stream())
+        return out_s, out_i
     call("pc_topk_by_type", dev(q, F32, "q"), rows, dim, dev(catalog, F32, "catalog"), dev(members, I32, "members"),
          dev(type_offsets, I64, "type_offsets"), int(n_types), dev(row_type, I32, "row_type"), k, splits, int(index_base),
          dev(out_s, F64, "out_scores"), dev(out_i, I64, "out_idx"), dev(ws, torch.uint8, "ws"), ws.numel(), stream())
@@ -853,10 +872,14 @@ def topk_by_type(q: torch.Tensor, catalog: torch.Tensor, type_offsets: torch.Ten
 
 def rank_by_type(q: torch.Tensor, catalog: torch.Tensor, type_offsets: torch.Tensor, n_types: int,
                  row_type: Optional[torch.Tensor], target_rows: torch.Tensor, target_idx: torch.Tensor,
-                 members: Optional[torch.Tensor] = None, index_base: int = 0, splits: Optional[int] = None) -> torch.Tensor:
+                 members: Optional[torch.Tensor] = None, index_base: int = 0, splits: Optional[int] = None,
+                 exclude=None, type_id: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Rank of each row's target among the catalog rows of the row's type (pc_rank_by_type): the number of products
     whose (score, global index) ranks strictly before (q[r] . target_rows[r], target_idx[r]); -1 for a row_type
-    outside [0, n_types).  Membership of the target is the caller's: the kernel does not check it.  Returns int64 [R]."""
+    outside [0, n_types).  Membership of the target is the caller's: the kernel does not check it.  Returns int64 [R].
+    exclude (retrieval.Exclusions of global indices): products of row r's list are not counted, the target itself
+    excepted (pc_rank_remove_excluded after the count; type_id int32 [P] is the catalog's local type of each row and
+    is needed with row_type)."""
     q = q.contiguous()
     rows, dim = q.shape
     target_rows = target_rows.contiguous()
@@ -880,6 +903,13 @@ def rank_by_type(q: torch.Tensor, catalog: torch.Tensor, type_offsets: torch.Ten
          dev(type_offsets, I64, "type_offsets"), int(n_types), dev(row_type, I32, "row_type"),
          dev(target_rows, F32, "target_rows"), dev(target_idx, I64, "target_idx"), splits, int(index_base),
          dev(out, I64, "out_rank"), dev(ws, torch.uint8, "ws"), ws.numel(), stream())
+    if exclude is not None:
+        if row_type is not None and type_id is None:
+            raise ValueError("rank_by_type: exclusions with row types need the catalog's type_id")
+        call("pc_rank_remove_excluded", dev(q, F32, "q"), rows, dim, dev(catalog, F32, "catalog"), catalog.shape[0],
+             dev(type_id if row_type is not None else None, I32, "type_id"), dev(row_type, I32, "row_type"),
+             dev(target_rows, F32, "target_rows"), dev(target_idx, I64, "target_idx"), int(index_base),
+             *_exclusion_args(exclude, rows, "rank_by_type"), dev(out, I64, "inout_rank"), stream())
     return out
 
 

@@ -11,6 +11,8 @@
 * ``ShardedCatalog`` shards the catalog rows over the ranks of a process group; each rank ranks
   its shard and the per-shard lists are all-gathered and merged (ties -> lowest global index);
   per-shard target ranks are added.
+* ``Exclusions`` are per-row lists of products a ranking leaves out (products a user already has, the query itself,
+  the other known positives of a filtered evaluation rank); they apply inside the top-K and rank kernels.
 """
 from __future__ import annotations
 
@@ -98,6 +100,121 @@ class Metrics:
         return metrics
 
 
+class Exclusions:
+    """Per-row exclusion lists for ``CatalogIndex.topk`` / ``rank`` / ``recommend`` and ``ShardedCatalog``: score row r
+    ignores the products of list E_r.
+
+    Lists hold GLOBAL product indices (int64) in CSR form: ``offsets`` [L + 1] and ``indices`` [offsets[L]], ascending
+    within each list (the constructor sorts them), duplicates allowed.  ``row_list`` [R] maps score row r to its list;
+    a value outside [0, L) means no exclusions; without row_list, row r uses list r.  Entries outside the catalog (or
+    shard) and entries of another type have no effect, so one set of lists serves every shard unchanged.
+
+    The input is validated once here (one host synchronisation, none per query): offsets[0] == 0, non-decreasing,
+    offsets[-1] == indices.numel(), row_list 1-D; anything else raises ValueError.  ``sorted=True`` skips the sort for
+    lists that are already ascending (a graph's CSR neighbour lists)."""
+
+    def __init__(self, offsets: torch.Tensor, indices: torch.Tensor, row_list: Optional[torch.Tensor] = None,
+                 sorted: bool = False):
+        offsets = torch.as_tensor(offsets)
+        indices = torch.as_tensor(indices, device=offsets.device)
+        if offsets.dim() != 1 or offsets.numel() < 1 or indices.dim() != 1:
+            raise ValueError(f"Exclusions: offsets {tuple(offsets.shape)} and indices {tuple(indices.shape)} must be 1-D, "
+                             "offsets with at least one entry")
+        if offsets.dtype.is_floating_point or indices.dtype.is_floating_point:
+            raise ValueError("Exclusions: offsets and indices must be integer tensors")
+        if offsets.numel() - 1 >= 2 ** 31:
+            raise ValueError(f"Exclusions: {offsets.numel() - 1} lists (at most 2^31 - 1)")
+        offsets = offsets.to(torch.int64).contiguous()
+        indices = indices.to(torch.int64).contiguous()
+        n = indices.numel()
+        ok = (offsets[0] == 0) & (offsets[-1] == n) & (offsets.diff() >= 0).all()
+        if not bool(ok):
+            raise ValueError("Exclusions: offsets must start at 0, be non-decreasing and end at indices.numel()")
+        if row_list is not None:
+            row_list = torch.as_tensor(row_list, device=offsets.device)
+            if row_list.dim() != 1 or row_list.dtype.is_floating_point:
+                raise ValueError(f"Exclusions: row_list {tuple(row_list.shape)} must be a 1-D integer tensor")
+        self.offsets = offsets
+        self.indices = indices if sorted else self._sort_lists(offsets, indices)
+        self.row_list = None if row_list is None else self._list_ids(row_list, self.num_lists)
+
+    @property
+    def num_lists(self) -> int:
+        return self.offsets.numel() - 1
+
+    @staticmethod
+    def _list_ids(row_list: torch.Tensor, n_lists: int) -> torch.Tensor:
+        """int32 list ids; anything outside [0, n_lists) becomes -1 (no exclusions) before the narrowing."""
+        rl = row_list.to(torch.int64)
+        return torch.where((rl >= 0) & (rl < n_lists), rl, torch.full_like(rl, -1)).to(torch.int32).contiguous()
+
+    @staticmethod
+    def _sort_lists(offsets: torch.Tensor, indices: torch.Tensor) -> torch.Tensor:
+        """Sort every list on the device: a stable sort by value, then a stable sort by list id."""
+        n = indices.numel()
+        if n == 0:
+            return indices
+        lid = torch.repeat_interleave(torch.arange(offsets.numel() - 1, device=offsets.device), offsets.diff(),
+                                      output_size=n)
+        by_value = torch.argsort(indices, stable=True)
+        by_list = torch.argsort(lid[by_value], stable=True)
+        return indices[by_value][by_list].contiguous()
+
+    @classmethod
+    def _trusted(cls, offsets: torch.Tensor, indices: torch.Tensor, row_list: Optional[torch.Tensor]) -> "Exclusions":
+        """Lists built by this module (valid offsets, ascending lists, int32 row_list): no validation, no sort."""
+        ex = cls.__new__(cls)
+        ex.offsets, ex.indices, ex.row_list = offsets, indices, row_list
+        return ex
+
+    @classmethod
+    def from_lists(cls, lists: Sequence[Sequence[int]], device, row_list: Optional[torch.Tensor] = None) -> "Exclusions":
+        """Lists of global product indices in any order (sorted on the device)."""
+        lens = torch.tensor([len(x) for x in lists], dtype=torch.int64)
+        offsets = torch.zeros(len(lists) + 1, dtype=torch.int64)
+        torch.cumsum(lens, 0, out=offsets[1:])
+        flat = torch.tensor([int(v) for x in lists for v in x], dtype=torch.int64)
+        return cls(offsets.to(device), flat.to(device), row_list)
+
+    def for_rows(self, row_of: torch.Tensor) -> "Exclusions":
+        """The same lists for new score rows, row i using the list of this object's row row_of[i] (no list is
+        copied)."""
+        row_of = row_of.to(self.offsets.device, torch.int64)
+        rl = self._list_ids(row_of, self.num_lists) if self.row_list is None else self.row_list[row_of].contiguous()
+        return Exclusions._trusted(self.offsets, self.indices, rl)
+
+    def union(self, other: "Exclusions", rows: int) -> "Exclusions":
+        """One list per score row r < rows: the union (with duplicates) of r's lists in self and in other."""
+        dev_ = self.offsets.device
+        beg_a, len_a = self._spans(rows)
+        beg_b, len_b = other._spans(rows)
+        lens = len_a + len_b
+        offsets = torch.zeros(rows + 1, dtype=torch.int64, device=dev_)
+        torch.cumsum(lens, 0, out=offsets[1:])
+        total = int(offsets[-1].item())
+        row = torch.repeat_interleave(torch.arange(rows, device=dev_), lens, output_size=total)
+        pos = torch.arange(total, device=dev_) - offsets[row]
+        src = torch.where(pos < len_a[row], beg_a[row] + pos, self.indices.numel() + beg_b[row] + pos - len_a[row])
+        values = torch.cat([self.indices, other.indices])[src]
+        return Exclusions._trusted(offsets, self._sort_lists(offsets, values), None)
+
+    def _spans(self, rows: int) -> Tuple[torch.Tensor, torch.Tensor]:
+        """(first entry, length) of the list of every score row r < rows (length 0 without a list)."""
+        dev_ = self.offsets.device
+        lid = self.row_list.to(torch.int64) if self.row_list is not None else torch.arange(rows, device=dev_)
+        if lid.numel() != rows:
+            raise ValueError(f"Exclusions: row_list has {lid.numel()} rows, expected {rows}")
+        ok = (lid >= 0) & (lid < self.num_lists)
+        safe = torch.where(ok, lid, torch.zeros_like(lid))
+        beg = self.offsets[safe]
+        return beg, torch.where(ok, self.offsets[safe + 1] - beg, torch.zeros_like(beg))
+
+
+def _check_exclusions(exclude: Optional[Exclusions], rows: int, what: str) -> None:
+    if exclude is not None and exclude.row_list is not None and exclude.row_list.numel() != rows:
+        raise ValueError(f"{what}: exclusion row_list has {exclude.row_list.numel()} entries for {rows} score rows")
+
+
 class CatalogIndex:
     """Type-segmented catalog on one GPU.
 
@@ -125,19 +242,22 @@ class CatalogIndex:
             self.num_types = n_types
 
     def topk(self, queries: torch.Tensor, k: int, row_type: Optional[torch.Tensor] = None,
-             splits: Optional[int] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+             splits: Optional[int] = None, exclude: Optional[Exclusions] = None) -> Tuple[torch.Tensor, torch.Tensor]:
         """Top-k per query row, 1 <= k <= ops.TOPK_MAX_K (1024; ValueError otherwise); row_type[r] restricts row r
         to products of that type (all products when row_type is None).  Returns (scores float64 [R, k], global
-        indices int64 [R, k]), padded with (-inf, -1) when a type has fewer than k products."""
+        indices int64 [R, k]), padded with (-inf, -1) when a type has fewer than k products.  exclude: row r ranks
+        its products without those of its exclusion list (the exact top-k of what remains)."""
         queries = queries.contiguous().float()
+        _check_exclusions(exclude, queries.shape[0], "CatalogIndex.topk")
         if row_type is None:
             if self._all is None:
                 self._all = torch.tensor([0, self.num_products], dtype=torch.int64, device=queries.device)
-            return ops.topk_by_type(queries, self.catalog, self._all, 1, None, k, None, self.index_base, splits)
+            return ops.topk_by_type(queries, self.catalog, self._all, 1, None, k, None, self.index_base, splits, exclude)
         if self.offsets is None:
             raise ValueError("CatalogIndex.topk: the catalog was built without type ids")
         rt = row_type.to(queries.device, torch.int32).contiguous()
-        return ops.topk_by_type(queries, self.catalog, self.offsets, self.num_types, rt, k, self.members, self.index_base, splits)
+        return ops.topk_by_type(queries, self.catalog, self.offsets, self.num_types, rt, k, self.members, self.index_base,
+                                splits, exclude)
 
     def topk_dense(self, queries: torch.Tensor, k: int, row_type: Optional[torch.Tensor] = None):
         """Same result as ``topk`` through the dense tensor-core path (BASELINE north_star part 4): single-pass TF32 scoring
@@ -176,8 +296,10 @@ class CatalogIndex:
         return rt, member, ops.gather_rows(self.catalog, safe)
 
     def _rank_counts(self, queries: torch.Tensor, target_rows: torch.Tensor, targets: torch.Tensor,
-                     row_type: Optional[torch.Tensor], splits: Optional[int] = None) -> torch.Tensor:
-        """Products of this catalog that rank before each target (pc_rank_by_type; -1 for a row type out of range)."""
+                     row_type: Optional[torch.Tensor], splits: Optional[int] = None,
+                     exclude: Optional[Exclusions] = None) -> torch.Tensor:
+        """Products of this catalog that rank before each target and are not excluded (pc_rank_by_type, then
+        pc_rank_remove_excluded; -1 for a row type out of range)."""
         targets = targets.to(queries.device, torch.int64).contiguous()
         if self.num_products == 0:
             return torch.zeros(queries.shape[0], dtype=torch.int64, device=queries.device)
@@ -185,28 +307,38 @@ class CatalogIndex:
             if self._all is None:
                 self._all = torch.tensor([0, self.num_products], dtype=torch.int64, device=queries.device)
             return ops.rank_by_type(queries, self.catalog, self._all, 1, None, target_rows, targets, None, self.index_base,
-                                    splits)
+                                    splits, exclude)
         return ops.rank_by_type(queries, self.catalog, self.offsets, self.num_types, row_type, target_rows, targets,
-                                self.members, self.index_base, splits)
+                                self.members, self.index_base, splits, exclude, self.type_id)
 
     def rank(self, queries: torch.Tensor, targets: torch.Tensor, row_type: Optional[torch.Tensor] = None,
-             splits: Optional[int] = None) -> torch.Tensor:
+             splits: Optional[int] = None, exclude: Optional[Exclusions] = None) -> torch.Tensor:
         """Exact rank of the product targets[r] (int64 global index) in row r's ranking: the number of products of the
         row's type (all products when row_type is None) that rank strictly before it, by score descending, then lower
         index.  -1 when the target can never be listed for the row: it is not in the catalog, or row_type[r] is not its
         type.  For every k, 0 <= rank < k exactly when ``topk(queries, k, row_type)`` lists the target, and it is then at
-        position rank.  Returns int64 [R]."""
+        position rank.  Returns int64 [R].
+
+        exclude: the "filtered" rank, which does not count the products of row r's exclusion list.  The target itself
+        is never removed, so a list of known positives can be passed as it is: 0 <= rank < k exactly when
+        ``topk(queries, k, row_type, exclude=E - {target})`` lists the target, at position rank."""
         queries = queries.contiguous().float()
+        _check_exclusions(exclude, queries.shape[0], "CatalogIndex.rank")
         rt, member, target_rows = self._owned_targets(queries, targets, row_type)
-        counts = self._rank_counts(queries, target_rows, targets, rt, splits)
+        counts = self._rank_counts(queries, target_rows, targets, rt, splits, exclude)
         return torch.where(member, counts, torch.full_like(counts, -1))
 
-    def recommend(self, projected_embeddings: torch.Tensor, complementary_types: torch.Tensor, k: int = 10):
+    def recommend(self, projected_embeddings: torch.Tensor, complementary_types: torch.Tensor, k: int = 10,
+                  exclude: Optional[Exclusions] = None):
         """The loop of inference.py:93-113 for a whole batch: projected [B, Kt, D], types [B, Kt] ->
         (scores [B, Kt, k], product indices [B, Kt, k]), 1 <= k <= ops.TOPK_MAX_K; a type with fewer than k products
-        pads its rows with (-inf, -1)."""
+        pads its rows with (-inf, -1).  exclude: lists per QUERY (row b of the batch, or exclude.row_list[b]); every
+        type row of query b leaves out query b's list."""
         b, kt, d = projected_embeddings.shape
-        s, i = self.topk(projected_embeddings.reshape(b * kt, d), k, complementary_types.reshape(-1))
+        if exclude is not None:
+            _check_exclusions(exclude, b, "CatalogIndex.recommend")
+            exclude = exclude.for_rows(torch.arange(b, device=projected_embeddings.device).repeat_interleave(kt))
+        s, i = self.topk(projected_embeddings.reshape(b * kt, d), k, complementary_types.reshape(-1), exclude=exclude)
         return s.reshape(b, kt, k), i.reshape(b, kt, k)
 
 
@@ -221,9 +353,12 @@ class ShardedCatalog:
         self.group = group
         self.local = CatalogIndex(local_catalog, local_type_id, index_base, num_types)
 
-    def topk(self, queries: torch.Tensor, k: int, row_type: Optional[torch.Tensor] = None):
+    def topk(self, queries: torch.Tensor, k: int, row_type: Optional[torch.Tensor] = None,
+             exclude: Optional[Exclusions] = None):
+        """CatalogIndex.topk over the whole sharded catalog; exclude holds global indices and every shard applies
+        the same lists."""
         import torch.distributed as dist
-        s, i = self.local.topk(queries, k, row_type)
+        s, i = self.local.topk(queries, k, row_type, exclude=exclude)
         world = dist.get_world_size(self.group) if dist.is_initialized() else 1
         if world == 1:
             return s, i
@@ -235,22 +370,24 @@ class ShardedCatalog:
         cat_i = gathered[:, :, k:].permute(1, 0, 2).reshape(s.shape[0], world * k).contiguous().view(torch.int64)
         return ops.topk_merge(cat_s, cat_i, k)
 
-    def rank(self, queries: torch.Tensor, targets: torch.Tensor, row_type: Optional[torch.Tensor] = None) -> torch.Tensor:
+    def rank(self, queries: torch.Tensor, targets: torch.Tensor, row_type: Optional[torch.Tensor] = None,
+             exclude: Optional[Exclusions] = None) -> torch.Tensor:
         """CatalogIndex.rank over the whole sharded catalog (queries, targets and row types replicated on every rank);
         equal to the rank on the unsharded catalog.  The shard that owns a target supplies its row and membership (one
         all-reduce: the other shards add zeros, which change no bit of the row), every shard counts its own products that
-        rank before it, and one all-reduce adds the counts."""
+        rank before it (less its own excluded products), and one all-reduce adds the counts."""
         import torch.distributed as dist
         world = dist.get_world_size(self.group) if dist.is_initialized() else 1
         if world == 1:
-            return self.local.rank(queries, targets, row_type)
+            return self.local.rank(queries, targets, row_type, exclude=exclude)
+        _check_exclusions(exclude, queries.shape[0], "ShardedCatalog.rank")
         queries = queries.contiguous().float()
         rt, member, target_rows = self.local._owned_targets(queries, targets, row_type)
         packed = torch.cat([torch.where(member[:, None], target_rows, torch.zeros_like(target_rows)),
                             member[:, None].float()], dim=1).contiguous()
         dist.all_reduce(packed, op=dist.ReduceOp.SUM, group=self.group)
         member = packed[:, -1] > 0
-        counts = self.local._rank_counts(queries, packed[:, :-1].contiguous(), targets, rt)
+        counts = self.local._rank_counts(queries, packed[:, :-1].contiguous(), targets, rt, exclude=exclude)
         counts = counts.clamp_min(0)               # a row type past this shard's type count: none of its products
         dist.all_reduce(counts, op=dist.ReduceOp.SUM, group=self.group)
         return torch.where(member, counts, torch.full_like(counts, -1))
