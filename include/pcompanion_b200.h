@@ -232,7 +232,7 @@ int pc_topk_groups(const float* q, int64_t rows, int dim, const float* catalog, 
  * [0, n_types) gives an all-padding row, as `if not type_products: continue` of inference.py:97-98.  Internally:
  * keys type << 32 | row, stable radix sort on the type bytes (pc_sort_keys), one pass that marks every eighth
  * row of a type's run as the start of a group (for k > 32: every row count the large-k kernel ranks in one
- * pass), then the pc_topk_groups kernel with one CTA row per position. */
+ * pass), then a ranking kernel with one CTA row per position that ranks each group as pc_topk_groups does. */
 size_t pc_topk_by_type_workspace_bytes(int64_t rows, int k, int splits);
 int pc_topk_by_type(const float* q, int64_t rows, int dim, const float* catalog, const int32_t* members,
                     const int64_t* type_offsets, int n_types, const int32_t* row_type, int k, int splits,
@@ -286,7 +286,7 @@ int pc_rank_remove_excluded(const float* q, int64_t rows, int dim, const float* 
  * GEMM (never materialised; approximate scores only select candidates), per-type mask (type_id[p] == row_type[r]; row_type NULL or < 0 = no mask) and a
  * per-row candidate list fused into the epilogue, then exact float64 re-scoring + ranking of the candidates.
  * `units` = product ranges per 128-row block (parallelism).  flags[r] = 1 when the guard band cannot prove
- * that no dropped product belongs to the top-k (the caller re-runs such rows on pc_topk_groups); results of
+ * that no dropped product belongs to the top-k (the caller re-runs such rows on pc_topk_by_type); results of
  * unflagged rows are identical to pc_topk_groups.  k <= 16, dim % 32 == 0, dim <= 128. */
 size_t pc_score_topk_workspace_bytes(int64_t rows, int units);
 int pc_score_topk_dense(const float* q, int64_t rows, int dim, const float* catalog, int64_t products,

@@ -15,6 +15,7 @@
 #include <math.h>
 
 #include <algorithm>
+#include <type_traits>
 
 #include "common.cuh"
 
@@ -98,6 +99,14 @@ constexpr int PP = 2;            // products per lane: every q value fetched fro
                                  // per SM cycle, fp64 pipe 24 % busy): 16 broadcast loads of q per 32 fp64 FMAs.
 constexpr int BATCH = 32 * PP;   // products per warp per pass
 constexpr int TILE_FLOATS = BATCH * TILE_LD;
+
+// [sb, se): split `split` of `splits` of the run [beg, end), in pieces of a multiple of 32 positions
+__device__ __forceinline__ void split_range(int64_t beg, int64_t end, int splits, int split, int64_t& sb, int64_t& se) {
+  const int64_t len = end > beg ? end - beg : 0;
+  const int64_t per = (ceil_div(len, int64_t(splits)) + 31) / 32 * 32;
+  sb = beg + per * split;
+  se = min(end, sb + per);
+}
 
 __device__ __forceinline__ void cp_async16(void* smem_dst, const void* gsrc, bool valid) {
   const uint32_t d = uint32_t(__cvta_generic_to_shared(smem_dst));
@@ -199,10 +208,8 @@ __device__ __forceinline__ void topk_group_body(const float* __restrict__ Q, int
     }
   }
   __syncthreads();
-  const int64_t len = end > beg ? end - beg : 0;
-  const int64_t per = (ceil_div(len, int64_t(splits)) + 31) / 32 * 32;
-  const int64_t sb = beg + per * split;
-  const int64_t se = min(end, sb + per);
+  int64_t sb, se;
+  split_range(beg, end, splits, split, sb, se);
   Cand mine[RB];
 #pragma unroll
   for (int r = 0; r < RB; ++r) mine[r] = Cand{-INFINITY, -1};
@@ -352,34 +359,21 @@ __global__ void topk_plan_kernel(const uint64_t* __restrict__ keys, int64_t rows
   grp_rows[p] = n;
 }
 
+// pc_topk_by_type's ranking kernel (k <= 32).  EXCL: with exclusion lists (pc_topk_by_type_excluding); the plain
+// instance ignores `ex`, which comes last so that the other parameters keep their offsets.
+template <bool EXCL>
 __global__ void __launch_bounds__(TK_WARPS * 32, 2)
 topk_planned_kernel(const float* __restrict__ Q, int dim, const float* __restrict__ catalog,
                     const int32_t* __restrict__ members, const int32_t* __restrict__ row_ids,
                     const int32_t* __restrict__ grp_rows, const uint64_t* __restrict__ keys,
                     const int64_t* __restrict__ type_offsets, int n_types, int64_t p0, int k, int splits,
-                    int64_t index_base, double* __restrict__ part_s, int64_t* __restrict__ part_i) {
+                    int64_t index_base, double* __restrict__ part_s, int64_t* __restrict__ part_i, const Excl ex) {
   const int64_t p = p0 + blockIdx.y;
   const int n_rows = grp_rows[p];
   if (n_rows == 0) return;                      // uniform over the CTA
   const int64_t t = int64_t(keys[p] >> 32);
   const int64_t beg = t < n_types ? type_offsets[t] : 0, end = t < n_types ? type_offsets[t + 1] : 0;
-  topk_group_body<false>(Q, dim, catalog, members, row_ids, int(p), n_rows, beg, end, k, splits, int(blockIdx.x), index_base,
-                         part_s, part_i, Excl{});
-}
-
-// topk_planned_kernel with exclusion lists (pc_topk_by_type_excluding, k <= 32)
-__global__ void __launch_bounds__(TK_WARPS * 32, 2)
-topk_planned_excl_kernel(const float* __restrict__ Q, int dim, const float* __restrict__ catalog,
-                         const int32_t* __restrict__ members, const int32_t* __restrict__ row_ids,
-                         const int32_t* __restrict__ grp_rows, const uint64_t* __restrict__ keys,
-                         const int64_t* __restrict__ type_offsets, int n_types, int64_t p0, int k, int splits,
-                         int64_t index_base, double* __restrict__ part_s, int64_t* __restrict__ part_i, const Excl ex) {
-  const int64_t p = p0 + blockIdx.y;
-  const int n_rows = grp_rows[p];
-  if (n_rows == 0) return;                      // uniform over the CTA
-  const int64_t t = int64_t(keys[p] >> 32);
-  const int64_t beg = t < n_types ? type_offsets[t] : 0, end = t < n_types ? type_offsets[t + 1] : 0;
-  topk_group_body<true>(Q, dim, catalog, members, row_ids, int(p), n_rows, beg, end, k, splits, int(blockIdx.x), index_base,
+  topk_group_body<EXCL>(Q, dim, catalog, members, row_ids, int(p), n_rows, beg, end, k, splits, int(blockIdx.x), index_base,
                         part_s, part_i, ex);
 }
 
@@ -563,10 +557,8 @@ __device__ __forceinline__ void topk_group_large_body(const float* __restrict__ 
     }
   }
   __syncthreads();
-  const int64_t len = end > beg ? end - beg : 0;
-  const int64_t per = (ceil_div(len, int64_t(splits)) + 31) / 32 * 32;
-  const int64_t sb = beg + per * split;
-  const int64_t se = min(end, sb + per);
+  int64_t sb, se;
+  split_range(beg, end, splits, split, sb, se);
   const int64_t n_pass = se > sb ? ceil_div(se - sb, int64_t(LK_GROUP_PASS)) : 0;
   float* tile = tiles + w * 2 * TILE_FLOATS;
   auto member_at = [&](int64_t pos) -> int { return pos < se ? (members ? members[pos] : int(pos)) : -1; };
@@ -631,37 +623,21 @@ topk_groups_large_kernel(const float* __restrict__ Q, int dim, const float* __re
                                   splits, int(blockIdx.x), index_base, part_s, part_i, Excl{});
 }
 
-// pc_topk_by_type's large-k ranking kernel: the plan formed groups of R rows, so one CTA ranks a whole group
-template <int R>
+// pc_topk_by_type's large-k ranking kernel: the plan formed groups of R rows, so one CTA ranks a whole group.  EXCL and
+// `ex` as topk_planned_kernel.
+template <int R, bool EXCL>
 __global__ void __launch_bounds__(LK_THREADS, 1)
 topk_planned_large_kernel(const float* __restrict__ Q, int dim, const float* __restrict__ catalog,
                           const int32_t* __restrict__ members, const int32_t* __restrict__ row_ids,
                           const int32_t* __restrict__ grp_rows, const uint64_t* __restrict__ keys,
                           const int64_t* __restrict__ type_offsets, int n_types, int64_t p0, int k, int cap, int splits,
-                          int64_t index_base, double* __restrict__ part_s, int64_t* __restrict__ part_i) {
+                          int64_t index_base, double* __restrict__ part_s, int64_t* __restrict__ part_i, const Excl ex) {
   const int64_t p = p0 + blockIdx.y;
   const int n_rows = grp_rows[p];
   if (n_rows == 0) return;                      // uniform over the CTA
   const int64_t t = int64_t(keys[p] >> 32);
   const int64_t beg = t < n_types ? type_offsets[t] : 0, end = t < n_types ? type_offsets[t + 1] : 0;
-  topk_group_large_body<R, false>(Q, dim, catalog, members, row_ids, int(p), n_rows, beg, end, k, cap, splits,
-                                  int(blockIdx.x), index_base, part_s, part_i, Excl{});
-}
-
-// topk_planned_large_kernel with exclusion lists (pc_topk_by_type_excluding, k > 32)
-template <int R>
-__global__ void __launch_bounds__(LK_THREADS, 1)
-topk_planned_large_excl_kernel(const float* __restrict__ Q, int dim, const float* __restrict__ catalog,
-                               const int32_t* __restrict__ members, const int32_t* __restrict__ row_ids,
-                               const int32_t* __restrict__ grp_rows, const uint64_t* __restrict__ keys,
-                               const int64_t* __restrict__ type_offsets, int n_types, int64_t p0, int k, int cap, int splits,
-                               int64_t index_base, double* __restrict__ part_s, int64_t* __restrict__ part_i, const Excl ex) {
-  const int64_t p = p0 + blockIdx.y;
-  const int n_rows = grp_rows[p];
-  if (n_rows == 0) return;                      // uniform over the CTA
-  const int64_t t = int64_t(keys[p] >> 32);
-  const int64_t beg = t < n_types ? type_offsets[t] : 0, end = t < n_types ? type_offsets[t + 1] : 0;
-  topk_group_large_body<R, true>(Q, dim, catalog, members, row_ids, int(p), n_rows, beg, end, k, cap, splits,
+  topk_group_large_body<R, EXCL>(Q, dim, catalog, members, row_ids, int(p), n_rows, beg, end, k, cap, splits,
                                  int(blockIdx.x), index_base, part_s, part_i, ex);
 }
 
@@ -735,6 +711,14 @@ int large_cap(int k, int pass) {
   return c;
 }
 
+constexpr size_t SMEM_BUDGET = 200 * 1024;   // most dynamic shared memory a group CTA may take (below the 227 KB per block)
+
+// k <= 32 group kernels: the staged queries, then the tile area that the candidate lists reuse
+size_t group_smem(int dim) {
+  return size_t(RB) * dim * sizeof(double) +
+         std::max(size_t(TK_WARPS) * 2 * TILE_FLOATS * sizeof(float), size_t(TK_WARPS) * RB * 32 * sizeof(Cand));
+}
+
 size_t group_large_smem(int rows, int cap, int dim) {
   return size_t(rows) * dim * sizeof(double) + size_t(TK_WARPS) * 2 * TILE_FLOATS * sizeof(float) +
          size_t(rows) * (cap + 1) * (sizeof(double) + sizeof(int32_t)) + size_t(rows) * sizeof(int);
@@ -743,76 +727,84 @@ size_t group_large_smem(int rows, int cap, int dim) {
 // score rows one large-k group CTA ranks per pass over its segment: the most (a power of two <= RB) whose buffers fit
 int group_large_rows(int cap, int dim) {
   int r = RB;
-  while (r > 1 && group_large_smem(r, cap, dim) > 200 * 1024) r >>= 1;
+  while (r > 1 && group_large_smem(r, cap, dim) > SMEM_BUDGET) r >>= 1;
   return r;
+}
+
+// f(std::integral_constant<int, R>) for R = group_large_rows(cap, dim): the large-k group kernels are built for R = 8/4/2/1
+template <typename F>
+int with_large_rows(int cap, int dim, F f) {
+  switch (group_large_rows(cap, dim)) {
+    case 8: return f(std::integral_constant<int, 8>{});
+    case 4: return f(std::integral_constant<int, 4>{});
+    case 2: return f(std::integral_constant<int, 2>{});
+    default: return f(std::integral_constant<int, 1>{});
+  }
 }
 
 size_t stream_smem_bytes(int cap) { return size_t(cap + 1) * (sizeof(double) + sizeof(int64_t)) + sizeof(int); }
 
-template <int R>
-int launch_groups_large(const float* q, int dim, const float* catalog, const int32_t* members, const int32_t* row_ids,
-                        const int32_t* grp_begin, const int64_t* seg_begin, const int64_t* seg_end, int64_t n_groups, int k,
-                        int cap, int splits, int64_t index_base, double* ps, int64_t* pi, cudaStream_t st) {
-  const size_t smem = group_large_smem(R, cap, dim);
-  PC_CUDA(cudaFuncSetAttribute(topk_groups_large_kernel<R>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-  for (int64_t g0 = 0; g0 < n_groups; g0 += 65535) {   // gridDim.y limit
-    const int64_t ng = n_groups - g0 < 65535 ? n_groups - g0 : 65535;
-    dim3 grid{unsigned(splits), unsigned(ng), unsigned(RB / R)};
-    topk_groups_large_kernel<R><<<grid, LK_THREADS, smem, st>>>(q, dim, catalog, members, row_ids, grp_begin + g0,
-                                                               seg_begin + g0, seg_end + g0, k, cap, splits, index_base, ps, pi);
+// gridDim.y is at most 65,535: launch(y0, ny) for every chunk [y0, y0 + ny) of the n rows or groups
+template <typename Launch>
+int launch_y_chunks(int64_t n, Launch launch) {
+  for (int64_t y0 = 0; y0 < n; y0 += 65535) {
+    launch(y0, unsigned(std::min<int64_t>(n - y0, 65535)));
     PC_LAUNCH_CHECK();
   }
   return PC_OK;
 }
 
-// ex == nullptr: no exclusion lists (topk_planned_large_kernel)
-template <int R>
-int launch_by_type_large(const float* q, int64_t rows, int dim, const float* catalog, const int32_t* members,
-                         const int64_t* type_offsets, int n_types, const uint64_t* keys, int32_t* row_ids, int32_t* grp_rows,
-                         int k, int cap, int splits, int64_t index_base, double* ps, int64_t* pi, const Excl* ex,
-                         cudaStream_t st) {
-  topk_plan_kernel<R><<<unsigned(ceil_div(rows, 256)), 256, 0, st>>>(keys, rows, row_ids, grp_rows);
+// With splits > 1, rank(ps, pi) writes every row's `splits` lists of k to split_ws ([rows][splits][k] scores, then the
+// indices) and pc_topk_merge reduces them to the output; with one split it writes the output directly.
+template <typename Rank>
+int with_split_lists(int64_t rows, int k, int splits, void* split_ws, double* out_scores, int64_t* out_idx,
+                     pc_stream_t stream, Rank rank) {
+  double* ps = out_scores;
+  int64_t* pi = out_idx;
+  if (splits > 1) {
+    ps = reinterpret_cast<double*>(split_ws);
+    pi = reinterpret_cast<int64_t*>(ps + size_t(rows) * splits * k);
+  }
+  if (int rc = rank(ps, pi)) return rc;
+  if (splits > 1) return pc_topk_merge(ps, pi, rows, splits, k, out_scores, out_idx, stream);
+  return PC_OK;
+}
+
+// The device-side grouping of pc_topk_by_type(_excluding) and pc_rank_by_type in the first by_type_plan_bytes(rows) of
+// the workspace: keys | sort workspace | row_ids | grp_rows.
+size_t by_type_plan_bytes(int64_t rows) {
+  if (rows <= 0) return 0;
+  return align_up(size_t(rows) * 8, 256) + align_up(pc_sort_keys_workspace_bytes(rows), 256) + 2 * align_up(size_t(rows) * 4, 256);
+}
+
+struct ByTypePlan {
+  const uint64_t* keys;
+  const int32_t* row_ids;
+  const int32_t* grp_rows;
+};
+
+// Sort the rows by type and mark groups of G rows (G: the rows per CTA of the ranking kernel that follows).
+template <int G>
+int plan_by_type(int64_t rows, int n_types, const int32_t* row_type, void* workspace, pc_stream_t stream, ByTypePlan& plan) {
+  cudaStream_t st = as_stream(stream);
+  char* ws = reinterpret_cast<char*>(workspace);
+  uint64_t* keys = reinterpret_cast<uint64_t*>(ws);             ws += align_up(size_t(rows) * 8, 256);
+  void* sort_ws = ws;                                            const size_t sort_bytes = pc_sort_keys_workspace_bytes(rows);
+  ws += align_up(sort_bytes, 256);
+  int32_t* row_ids = reinterpret_cast<int32_t*>(ws);             ws += align_up(size_t(rows) * 4, 256);
+  int32_t* grp_rows = reinterpret_cast<int32_t*>(ws);
+  const unsigned tb = unsigned(ceil_div(rows, 256));
+  type_keys_kernel<<<tb, 256, 0, st>>>(row_type, rows, n_types, keys);
   PC_LAUNCH_CHECK();
-  const size_t smem = group_large_smem(R, cap, dim) + (ex ? 8 + 2 * R * sizeof(int64_t) : 0);   // + aligned list bounds
-  if (ex) PC_CUDA(cudaFuncSetAttribute(topk_planned_large_excl_kernel<R>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-  else PC_CUDA(cudaFuncSetAttribute(topk_planned_large_kernel<R>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-  for (int64_t p0 = 0; p0 < rows; p0 += 65535) {   // gridDim.y limit
-    const int64_t np = rows - p0 < 65535 ? rows - p0 : 65535;
-    dim3 grid{unsigned(splits), unsigned(np), 1u};
-    if (ex)
-      topk_planned_large_excl_kernel<R><<<grid, LK_THREADS, smem, st>>>(q, dim, catalog, members, row_ids, grp_rows, keys,
-                                                                       type_offsets, n_types, p0, k, cap, splits, index_base,
-                                                                       ps, pi, *ex);
-    else
-      topk_planned_large_kernel<R><<<grid, LK_THREADS, smem, st>>>(q, dim, catalog, members, row_ids, grp_rows, keys,
-                                                                  type_offsets, n_types, p0, k, cap, splits, index_base, ps, pi);
-    PC_LAUNCH_CHECK();
-  }
+  // keys are created in ascending row order and the sort is stable: only the type bytes take part
+  uint32_t mask = 0;
+  for (int b = 0; b < 4; ++b)
+    if ((uint64_t(n_types) >> (8 * b)) != 0) mask |= 1u << (4 + b);
+  if (int rc = pc_sort_keys(keys, rows, mask, sort_ws, sort_bytes, stream)) return rc;
+  topk_plan_kernel<G><<<tb, 256, 0, st>>>(keys, rows, row_ids, grp_rows);
+  PC_LAUNCH_CHECK();
+  plan = ByTypePlan{keys, row_ids, grp_rows};
   return PC_OK;
-}
-
-int groups_large(const float* q, int dim, const float* catalog, const int32_t* members, const int32_t* row_ids,
-                 const int32_t* grp_begin, const int64_t* seg_begin, const int64_t* seg_end, int64_t n_groups, int k,
-                 int splits, int64_t index_base, double* ps, int64_t* pi, cudaStream_t st) {
-  const int cap = large_cap(k, LK_GROUP_PASS);
-  switch (group_large_rows(cap, dim)) {
-    case 8: return launch_groups_large<8>(q, dim, catalog, members, row_ids, grp_begin, seg_begin, seg_end, n_groups, k, cap, splits, index_base, ps, pi, st);
-    case 4: return launch_groups_large<4>(q, dim, catalog, members, row_ids, grp_begin, seg_begin, seg_end, n_groups, k, cap, splits, index_base, ps, pi, st);
-    case 2: return launch_groups_large<2>(q, dim, catalog, members, row_ids, grp_begin, seg_begin, seg_end, n_groups, k, cap, splits, index_base, ps, pi, st);
-    default: return launch_groups_large<1>(q, dim, catalog, members, row_ids, grp_begin, seg_begin, seg_end, n_groups, k, cap, splits, index_base, ps, pi, st);
-  }
-}
-
-int by_type_large(const float* q, int64_t rows, int dim, const float* catalog, const int32_t* members,
-                  const int64_t* type_offsets, int n_types, const uint64_t* keys, int32_t* row_ids, int32_t* grp_rows, int k,
-                  int splits, int64_t index_base, double* ps, int64_t* pi, const Excl* ex, cudaStream_t st) {
-  const int cap = large_cap(k, LK_GROUP_PASS);
-  switch (group_large_rows(cap, dim)) {
-    case 8: return launch_by_type_large<8>(q, rows, dim, catalog, members, type_offsets, n_types, keys, row_ids, grp_rows, k, cap, splits, index_base, ps, pi, ex, st);
-    case 4: return launch_by_type_large<4>(q, rows, dim, catalog, members, type_offsets, n_types, keys, row_ids, grp_rows, k, cap, splits, index_base, ps, pi, ex, st);
-    case 2: return launch_by_type_large<2>(q, rows, dim, catalog, members, type_offsets, n_types, keys, row_ids, grp_rows, k, cap, splits, index_base, ps, pi, ex, st);
-    default: return launch_by_type_large<1>(q, rows, dim, catalog, members, type_offsets, n_types, keys, row_ids, grp_rows, k, cap, splits, index_base, ps, pi, ex, st);
-  }
 }
 
 // ---- rank of a target (pc_rank_by_type).  The rank of row r's target is the number of products of the row's run that
@@ -863,11 +855,8 @@ rank_planned_kernel(const float* __restrict__ Q, int dim, const float* __restric
     tgt_i[r] = g;
   }
   __syncthreads();
-  const int64_t beg = type_offsets[t], end = type_offsets[t + 1];
-  const int64_t len = end > beg ? end - beg : 0;
-  const int64_t per = (ceil_div(len, int64_t(splits)) + 31) / 32 * 32;
-  const int64_t sb = beg + per * blockIdx.x;
-  const int64_t se = min(end, sb + per);
+  int64_t sb, se;
+  split_range(type_offsets[t], type_offsets[t + 1], splits, int(blockIdx.x), sb, se);
   float* tile = tiles + w * 2 * TILE_FLOATS;
   auto member_at = [&](int64_t pos) -> int { return pos < se ? (members ? members[pos] : int(pos)) : -1; };
 
@@ -977,47 +966,44 @@ extern "C" int pc_topk_groups(const float* q, int64_t rows, int dim, const float
   PC_REQUIRE(k >= 1 && k <= PC_TOPK_MAX_K, PC_ERR_UNSUPPORTED, "topk_groups: k=%d outside [1,%d]", k, PC_TOPK_MAX_K);
   PC_REQUIRE(dim >= DCH && dim % DCH == 0 && dim <= 1024, PC_ERR_UNSUPPORTED, "topk_groups: dim=%d must be a multiple of %d (<= 1024)", dim, DCH);
   PC_REQUIRE(splits >= 1 && splits <= 65535, PC_ERR_UNSUPPORTED, "topk_groups: bad splits");
+  PC_REQUIRE(splits == 1 || (workspace && workspace_bytes >= pc_topk_groups_workspace_bytes(rows, k, splits)),
+             PC_ERR_WORKSPACE, "topk_groups: workspace too small");
   cudaStream_t st = as_stream(stream);
-  const size_t smem = size_t(RB) * dim * sizeof(double) +
-                      std::max(size_t(TK_WARPS) * 2 * TILE_FLOATS * sizeof(float), size_t(TK_WARPS) * RB * 32 * sizeof(Cand));
-  PC_CUDA(cudaFuncSetAttribute(topk_groups_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-  PC_REQUIRE(smem <= 200 * 1024, PC_ERR_UNSUPPORTED, "topk_groups: shared memory budget exceeded");
-  double* ps = out_scores;
-  int64_t* pi = out_idx;
-  if (splits > 1) {
-    PC_REQUIRE(workspace && workspace_bytes >= pc_topk_groups_workspace_bytes(rows, k, splits), PC_ERR_WORKSPACE,
-               "topk_groups: workspace too small");
-    ps = reinterpret_cast<double*>(workspace);
-    pi = reinterpret_cast<int64_t*>(ps + size_t(rows) * splits * k);
-  }
-  if (k > WARP_K) {
-    if (int rc = groups_large(q, dim, catalog, members, row_ids, grp_begin, seg_begin, seg_end, n_groups, k, splits,
-                              index_base, ps, pi, st))
-      return rc;
-  } else {
-    for (int64_t g0 = 0; g0 < n_groups; g0 += 65535) {   // gridDim.y limit
-      const int64_t ng = n_groups - g0 < 65535 ? n_groups - g0 : 65535;
-      dim3 grid{unsigned(splits), unsigned(ng), 1u};
-      topk_groups_kernel<<<grid, TK_WARPS * 32, smem, st>>>(q, dim, catalog, members, row_ids, grp_begin + g0, seg_begin + g0,
-                                                            seg_end + g0, k, splits, index_base, ps, pi);
-      PC_LAUNCH_CHECK();
+  return with_split_lists(rows, k, splits, workspace, out_scores, out_idx, stream, [&](double* ps, int64_t* pi) -> int {
+    if (k > WARP_K) {
+      const int cap = large_cap(k, LK_GROUP_PASS);
+      return with_large_rows(cap, dim, [&](auto rows_per_cta) -> int {
+        constexpr int R = decltype(rows_per_cta)::value;
+        const size_t smem = group_large_smem(R, cap, dim);
+        PC_CUDA(cudaFuncSetAttribute(topk_groups_large_kernel<R>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+        return launch_y_chunks(n_groups, [&](int64_t g0, unsigned ng) {
+          topk_groups_large_kernel<R><<<dim3(splits, ng, RB / R), LK_THREADS, smem, st>>>(
+              q, dim, catalog, members, row_ids, grp_begin + g0, seg_begin + g0, seg_end + g0, k, cap, splits, index_base,
+              ps, pi);
+        });
+      });
     }
-  }
-  if (splits > 1) return pc_topk_merge(ps, pi, rows, splits, k, out_scores, out_idx, stream);
-  return PC_OK;
+    const size_t smem = group_smem(dim);
+    PC_CUDA(cudaFuncSetAttribute(topk_groups_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(SMEM_BUDGET)));
+    PC_REQUIRE(smem <= SMEM_BUDGET, PC_ERR_UNSUPPORTED, "topk_groups: shared memory budget exceeded");
+    return launch_y_chunks(n_groups, [&](int64_t g0, unsigned ng) {
+      topk_groups_kernel<<<dim3(splits, ng, 1), TK_WARPS * 32, smem, st>>>(q, dim, catalog, members, row_ids, grp_begin + g0,
+                                                                          seg_begin + g0, seg_end + g0, k, splits, index_base,
+                                                                          ps, pi);
+    });
+  });
 }
 
 extern "C" size_t pc_topk_by_type_workspace_bytes(int64_t rows, int k, int splits) {
-  if (rows <= 0) return 0;
-  return align_up(size_t(rows) * 8, 256) + align_up(pc_sort_keys_workspace_bytes(rows), 256) + 2 * align_up(size_t(rows) * 4, 256) +
-         pc_topk_groups_workspace_bytes(rows, k, splits);
+  return by_type_plan_bytes(rows) + pc_topk_groups_workspace_bytes(rows, k, splits);
 }
 
-// pc_topk_by_type (ex == nullptr) and pc_topk_by_type_excluding: the same grouping, splits and merge
+// pc_topk_by_type (EXCL = false, `ex` ignored) and pc_topk_by_type_excluding: the same grouping, splits and merge
+template <bool EXCL>
 static int topk_by_type_impl(const float* q, int64_t rows, int dim, const float* catalog, const int32_t* members,
                              const int64_t* type_offsets, int n_types, const int32_t* row_type, int k, int splits,
                              int64_t index_base, double* out_scores, int64_t* out_idx, void* workspace,
-                             size_t workspace_bytes, const Excl* ex, pc_stream_t stream) {
+                             size_t workspace_bytes, const Excl ex, pc_stream_t stream) {
   PC_REQUIRE(rows >= 0 && rows < (int64_t(1) << 31), PC_ERR_INVALID, "topk_by_type: bad row count");
   if (rows == 0) return PC_OK;
   PC_REQUIRE(q && catalog && type_offsets && out_scores && out_idx && workspace, PC_ERR_INVALID, "topk_by_type: null pointer");
@@ -1027,60 +1013,42 @@ static int topk_by_type_impl(const float* q, int64_t rows, int dim, const float*
   PC_REQUIRE(splits >= 1 && splits <= 65535, PC_ERR_UNSUPPORTED, "topk_by_type: bad splits");
   PC_REQUIRE(workspace_bytes >= pc_topk_by_type_workspace_bytes(rows, k, splits), PC_ERR_WORKSPACE, "topk_by_type: workspace too small");
   cudaStream_t st = as_stream(stream);
-  char* ws = reinterpret_cast<char*>(workspace);
-  uint64_t* keys = reinterpret_cast<uint64_t*>(ws);             ws += align_up(size_t(rows) * 8, 256);
-  void* sort_ws = ws;                                            const size_t sort_bytes = pc_sort_keys_workspace_bytes(rows);
-  ws += align_up(sort_bytes, 256);
-  int32_t* row_ids = reinterpret_cast<int32_t*>(ws);             ws += align_up(size_t(rows) * 4, 256);
-  int32_t* grp_rows = reinterpret_cast<int32_t*>(ws);            ws += align_up(size_t(rows) * 4, 256);
-  const unsigned tb = unsigned(ceil_div(rows, 256));
-  type_keys_kernel<<<tb, 256, 0, st>>>(row_type, rows, n_types, keys);
-  PC_LAUNCH_CHECK();
-  // keys are created in ascending row order and the sort is stable: only the type bytes take part
-  uint32_t mask = 0;
-  for (int b = 0; b < 4; ++b)
-    if ((uint64_t(n_types) >> (8 * b)) != 0) mask |= 1u << (4 + b);
-  if (int rc = pc_sort_keys(keys, rows, mask, sort_ws, sort_bytes, stream)) return rc;
-  double* ps = out_scores;
-  int64_t* pi = out_idx;
-  if (splits > 1) {
-    ps = reinterpret_cast<double*>(ws);
-    pi = reinterpret_cast<int64_t*>(ps + size_t(rows) * splits * k);
-  }
-  if (k > WARP_K) {
-    if (int rc = by_type_large(q, rows, dim, catalog, members, type_offsets, n_types, keys, row_ids, grp_rows, k, splits,
-                               index_base, ps, pi, ex, st))
-      return rc;
-  } else {
-    topk_plan_kernel<RB><<<tb, 256, 0, st>>>(keys, rows, row_ids, grp_rows);
-    PC_LAUNCH_CHECK();
-    const size_t smem = size_t(RB) * dim * sizeof(double) +
-                        std::max(size_t(TK_WARPS) * 2 * TILE_FLOATS * sizeof(float), size_t(TK_WARPS) * RB * 32 * sizeof(Cand));
-    PC_REQUIRE(smem <= 200 * 1024, PC_ERR_UNSUPPORTED, "topk_by_type: shared memory budget exceeded");
-    if (ex) PC_CUDA(cudaFuncSetAttribute(topk_planned_excl_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    else PC_CUDA(cudaFuncSetAttribute(topk_planned_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    for (int64_t p0 = 0; p0 < rows; p0 += 65535) {   // gridDim.y limit
-      const int64_t np = rows - p0 < 65535 ? rows - p0 : 65535;
-      dim3 grid{unsigned(splits), unsigned(np), 1u};
-      if (ex)   // + the rows' list bounds after the tile area
-        topk_planned_excl_kernel<<<grid, TK_WARPS * 32, smem + 2 * RB * sizeof(int64_t), st>>>(
-            q, dim, catalog, members, row_ids, grp_rows, keys, type_offsets, n_types, p0, k, splits, index_base, ps, pi, *ex);
-      else
-        topk_planned_kernel<<<grid, TK_WARPS * 32, smem, st>>>(q, dim, catalog, members, row_ids, grp_rows, keys, type_offsets,
-                                                               n_types, p0, k, splits, index_base, ps, pi);
-      PC_LAUNCH_CHECK();
+  void* split_ws = reinterpret_cast<char*>(workspace) + by_type_plan_bytes(rows);
+  return with_split_lists(rows, k, splits, split_ws, out_scores, out_idx, stream, [&](double* ps, int64_t* pi) -> int {
+    ByTypePlan plan;
+    if (k > WARP_K) {
+      const int cap = large_cap(k, LK_GROUP_PASS);
+      return with_large_rows(cap, dim, [&](auto rows_per_cta) -> int {
+        constexpr int R = decltype(rows_per_cta)::value;
+        if (int rc = plan_by_type<R>(rows, n_types, row_type, workspace, stream, plan)) return rc;
+        const size_t smem = group_large_smem(R, cap, dim) + (EXCL ? 8 + 2 * R * sizeof(int64_t) : 0);   // + aligned list bounds
+        PC_CUDA(cudaFuncSetAttribute(topk_planned_large_kernel<R, EXCL>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+        return launch_y_chunks(rows, [&](int64_t p0, unsigned np) {
+          topk_planned_large_kernel<R, EXCL><<<dim3(splits, np, 1), LK_THREADS, smem, st>>>(
+              q, dim, catalog, members, plan.row_ids, plan.grp_rows, plan.keys, type_offsets, n_types, p0, k, cap, splits,
+              index_base, ps, pi, ex);
+        });
+      });
     }
-  }
-  if (splits > 1) return pc_topk_merge(ps, pi, rows, splits, k, out_scores, out_idx, stream);
-  return PC_OK;
+    if (int rc = plan_by_type<RB>(rows, n_types, row_type, workspace, stream, plan)) return rc;
+    const size_t smem = group_smem(dim);
+    PC_REQUIRE(smem <= SMEM_BUDGET, PC_ERR_UNSUPPORTED, "topk_by_type: shared memory budget exceeded");
+    PC_CUDA(cudaFuncSetAttribute(topk_planned_kernel<EXCL>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(SMEM_BUDGET)));
+    const size_t smem_ex = smem + (EXCL ? 2 * RB * sizeof(int64_t) : 0);   // + the rows' list bounds after the tile area
+    return launch_y_chunks(rows, [&](int64_t p0, unsigned np) {
+      topk_planned_kernel<EXCL><<<dim3(splits, np, 1), TK_WARPS * 32, smem_ex, st>>>(
+          q, dim, catalog, members, plan.row_ids, plan.grp_rows, plan.keys, type_offsets, n_types, p0, k, splits, index_base,
+          ps, pi, ex);
+    });
+  });
 }
 
 extern "C" int pc_topk_by_type(const float* q, int64_t rows, int dim, const float* catalog, const int32_t* members,
                                const int64_t* type_offsets, int n_types, const int32_t* row_type, int k, int splits,
                                int64_t index_base, double* out_scores, int64_t* out_idx, void* workspace,
                                size_t workspace_bytes, pc_stream_t stream) {
-  return topk_by_type_impl(q, rows, dim, catalog, members, type_offsets, n_types, row_type, k, splits, index_base,
-                           out_scores, out_idx, workspace, workspace_bytes, nullptr, stream);
+  return topk_by_type_impl<false>(q, rows, dim, catalog, members, type_offsets, n_types, row_type, k, splits, index_base,
+                                  out_scores, out_idx, workspace, workspace_bytes, Excl{}, stream);
 }
 
 extern "C" int pc_topk_by_type_excluding(const float* q, int64_t rows, int dim, const float* catalog, const int32_t* members,
@@ -1091,14 +1059,11 @@ extern "C" int pc_topk_by_type_excluding(const float* q, int64_t rows, int dim, 
   PC_REQUIRE(n_lists >= 0, PC_ERR_INVALID, "topk_by_type_excluding: n_lists=%lld < 0", (long long)n_lists);
   PC_REQUIRE(n_lists == 0 || (excl_offsets && excl_idx), PC_ERR_INVALID, "topk_by_type_excluding: null exclusion lists");
   const Excl ex{excl_offsets, excl_idx, n_lists, row_list};
-  return topk_by_type_impl(q, rows, dim, catalog, members, type_offsets, n_types, row_type, k, splits, index_base,
-                           out_scores, out_idx, workspace, workspace_bytes, &ex, stream);
+  return topk_by_type_impl<true>(q, rows, dim, catalog, members, type_offsets, n_types, row_type, k, splits, index_base,
+                                 out_scores, out_idx, workspace, workspace_bytes, ex, stream);
 }
 
-extern "C" size_t pc_rank_by_type_workspace_bytes(int64_t rows) {
-  if (rows <= 0) return 0;
-  return align_up(size_t(rows) * 8, 256) + align_up(pc_sort_keys_workspace_bytes(rows), 256) + 2 * align_up(size_t(rows) * 4, 256);
-}
+extern "C" size_t pc_rank_by_type_workspace_bytes(int64_t rows) { return by_type_plan_bytes(rows); }
 
 extern "C" int pc_rank_by_type(const float* q, int64_t rows, int dim, const float* catalog, const int32_t* members,
                                const int64_t* type_offsets, int n_types, const int32_t* row_type, const float* target_rows,
@@ -1113,34 +1078,17 @@ extern "C" int pc_rank_by_type(const float* q, int64_t rows, int dim, const floa
   PC_REQUIRE(splits >= 1 && splits <= 65535, PC_ERR_UNSUPPORTED, "rank_by_type: bad splits");
   PC_REQUIRE(workspace_bytes >= pc_rank_by_type_workspace_bytes(rows), PC_ERR_WORKSPACE, "rank_by_type: workspace too small");
   cudaStream_t st = as_stream(stream);
-  char* ws = reinterpret_cast<char*>(workspace);
-  uint64_t* keys = reinterpret_cast<uint64_t*>(ws);             ws += align_up(size_t(rows) * 8, 256);
-  void* sort_ws = ws;                                            const size_t sort_bytes = pc_sort_keys_workspace_bytes(rows);
-  ws += align_up(sort_bytes, 256);
-  int32_t* row_ids = reinterpret_cast<int32_t*>(ws);             ws += align_up(size_t(rows) * 4, 256);
-  int32_t* grp_rows = reinterpret_cast<int32_t*>(ws);
   PC_CUDA(cudaMemsetAsync(out_rank, 0, size_t(rows) * sizeof(int64_t), st));
-  const unsigned tb = unsigned(ceil_div(rows, 256));
-  type_keys_kernel<<<tb, 256, 0, st>>>(row_type, rows, n_types, keys);
-  PC_LAUNCH_CHECK();
-  uint32_t mask = 0;
-  for (int b = 0; b < 4; ++b)
-    if ((uint64_t(n_types) >> (8 * b)) != 0) mask |= 1u << (4 + b);
-  if (int rc = pc_sort_keys(keys, rows, mask, sort_ws, sort_bytes, stream)) return rc;
-  topk_plan_kernel<RB><<<tb, 256, 0, st>>>(keys, rows, row_ids, grp_rows);
-  PC_LAUNCH_CHECK();
+  ByTypePlan plan;
+  if (int rc = plan_by_type<RB>(rows, n_types, row_type, workspace, stream, plan)) return rc;
   const size_t smem = size_t(RB) * dim * sizeof(double) + size_t(TK_WARPS) * 2 * TILE_FLOATS * sizeof(float) +
                       size_t(RB) * (sizeof(double) + sizeof(int64_t) + sizeof(unsigned long long));
   PC_CUDA(cudaFuncSetAttribute(rank_planned_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-  for (int64_t p0 = 0; p0 < rows; p0 += 65535) {   // gridDim.y limit
-    const int64_t np = rows - p0 < 65535 ? rows - p0 : 65535;
-    dim3 grid{unsigned(splits), unsigned(np), 1u};
-    rank_planned_kernel<<<grid, TK_WARPS * 32, smem, st>>>(q, dim, catalog, members, row_ids, grp_rows, keys, type_offsets,
-                                                           n_types, p0, target_rows, target_idx, splits, index_base,
-                                                           reinterpret_cast<unsigned long long*>(out_rank));
-    PC_LAUNCH_CHECK();
-  }
-  return PC_OK;
+  return launch_y_chunks(rows, [&](int64_t p0, unsigned np) {
+    rank_planned_kernel<<<dim3(splits, np, 1), TK_WARPS * 32, smem, st>>>(
+        q, dim, catalog, members, plan.row_ids, plan.grp_rows, plan.keys, type_offsets, n_types, p0, target_rows, target_idx,
+        splits, index_base, reinterpret_cast<unsigned long long*>(out_rank));
+  });
 }
 
 extern "C" int pc_rank_remove_excluded(const float* q, int64_t rows, int dim, const float* catalog, int64_t n_products,
@@ -1192,28 +1140,20 @@ extern "C" int pc_topk_rows(const float* values, int64_t rows, int64_t cols, int
   PC_REQUIRE(values && out_scores && out_idx, PC_ERR_INVALID, "topk_rows: null pointer");
   PC_REQUIRE(k >= 1 && k <= PC_TOPK_MAX_K, PC_ERR_UNSUPPORTED, "topk_rows: k=%d outside [1,%d]", k, PC_TOPK_MAX_K);
   PC_REQUIRE(splits >= 1 && splits <= 65535, PC_ERR_UNSUPPORTED, "topk_rows: bad splits");
+  PC_REQUIRE(splits == 1 || (workspace && workspace_bytes >= pc_topk_rows_workspace_bytes(rows, k, splits)),
+             PC_ERR_WORKSPACE, "topk_rows: workspace too small");
   cudaStream_t st = as_stream(stream);
-  double* ps = out_scores;
-  int64_t* pi = out_idx;
-  if (splits > 1) {
-    PC_REQUIRE(workspace && workspace_bytes >= pc_topk_rows_workspace_bytes(rows, k, splits), PC_ERR_WORKSPACE,
-               "topk_rows: workspace too small");
-    ps = reinterpret_cast<double*>(workspace);
-    pi = reinterpret_cast<int64_t*>(ps + size_t(rows) * splits * k);
-  }
-  for (int64_t r0 = 0; r0 < rows; r0 += 65535) {
-    const int64_t nr = rows - r0 < 65535 ? rows - r0 : 65535;
-    dim3 grid{unsigned(splits), unsigned(nr), 1u};
-    if (k > WARP_K) {
-      const int cap = large_cap(k, LK_STREAM_PASS);
-      topk_values_large_kernel<<<grid, LK_THREADS, stream_smem_bytes(cap), st>>>(values + r0 * cols, cols, k, cap, splits,
-                                                                                ps + r0 * splits * k, pi + r0 * splits * k);
-    } else {
-      topk_values_kernel<<<grid, TK_WARPS * 32, 0, st>>>(values + r0 * cols, cols, k, splits, ps + r0 * splits * k,
-                                                         pi + r0 * splits * k);
-    }
-    PC_LAUNCH_CHECK();
-  }
-  if (splits > 1) return pc_topk_merge(ps, pi, rows, splits, k, out_scores, out_idx, stream);
-  return PC_OK;
+  return with_split_lists(rows, k, splits, workspace, out_scores, out_idx, stream, [&](double* ps, int64_t* pi) {
+    return launch_y_chunks(rows, [&](int64_t r0, unsigned nr) {
+      const dim3 grid{unsigned(splits), nr, 1u};
+      if (k > WARP_K) {
+        const int cap = large_cap(k, LK_STREAM_PASS);
+        topk_values_large_kernel<<<grid, LK_THREADS, stream_smem_bytes(cap), st>>>(values + r0 * cols, cols, k, cap, splits,
+                                                                                  ps + r0 * splits * k, pi + r0 * splits * k);
+      } else {
+        topk_values_kernel<<<grid, TK_WARPS * 32, 0, st>>>(values + r0 * cols, cols, k, splits, ps + r0 * splits * k,
+                                                           pi + r0 * splits * k);
+      }
+    });
+  });
 }

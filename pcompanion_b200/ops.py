@@ -827,6 +827,14 @@ def topk_segments(q: torch.Tensor, catalog: torch.Tensor, seg_begin: torch.Tenso
     return out_s, out_i
 
 
+def _by_type_splits(rows: int, n_types: int, catalog: torch.Tensor, members: Optional[torch.Tensor], k: int = 1) -> int:
+    """Automatic splits of the device-grouped calls (topk_by_type, rank_by_type)."""
+    # expected number of groups without looking at the data: distinct types hit + one more group per 8 rows
+    n_cat = members.numel() if members is not None else catalog.shape[0]
+    distinct = n_types * (1.0 - math.exp(-rows / max(n_types, 1)))
+    return _auto_splits(int(distinct + rows / TOPK_GROUP_ROWS) + 1, n_cat / max(n_types, 1), k, rows)
+
+
 def _exclusion_args(exclude, rows: int, what: str):
     """(excl_offsets, excl_idx, n_lists, row_list) pointers of a retrieval.Exclusions for `rows` score rows."""
     if exclude.row_list is not None and tuple(exclude.row_list.shape) != (rows,):
@@ -853,10 +861,7 @@ def topk_by_type(q: torch.Tensor, catalog: torch.Tensor, type_offsets: torch.Ten
     if rows == 0:
         return out_s, out_i
     if splits is None:
-        # expected number of groups without looking at the data: distinct types hit + one more group per 8 rows
-        n_cat = members.numel() if members is not None else catalog.shape[0]
-        distinct = n_types * (1.0 - math.exp(-rows / max(n_types, 1)))
-        splits = _auto_splits(int(distinct + rows / TOPK_GROUP_ROWS) + 1, n_cat / max(n_types, 1), k, rows)
+        splits = _by_type_splits(rows, n_types, catalog, members, k)
     ws = _lib.workspace(_lib.LIB.pc_topk_by_type_workspace_bytes(rows, k, splits), q.device)
     if exclude is not None:
         call("pc_topk_by_type_excluding", dev(q, F32, "q"), rows, dim, dev(catalog, F32, "catalog"),
@@ -894,10 +899,7 @@ def rank_by_type(q: torch.Tensor, catalog: torch.Tensor, type_offsets: torch.Ten
     if rows == 0:
         return out
     if splits is None:
-        # as topk_by_type for k <= 32
-        n_cat = members.numel() if members is not None else catalog.shape[0]
-        distinct = n_types * (1.0 - math.exp(-rows / max(n_types, 1)))
-        splits = _auto_splits(int(distinct + rows / TOPK_GROUP_ROWS) + 1, n_cat / max(n_types, 1))
+        splits = _by_type_splits(rows, n_types, catalog, members)   # as topk_by_type for k <= 32
     ws = _lib.workspace(_lib.LIB.pc_rank_by_type_workspace_bytes(rows), q.device)
     call("pc_rank_by_type", dev(q, F32, "q"), rows, dim, dev(catalog, F32, "catalog"), dev(members, I32, "members"),
          dev(type_offsets, I64, "type_offsets"), int(n_types), dev(row_type, I32, "row_type"),
@@ -917,7 +919,7 @@ def score_topk_dense(q: torch.Tensor, catalog: torch.Tensor, k: int, type_id: Op
                      row_type: Optional[torch.Tensor] = None, index_base: int = 0, max_norm: Optional[float] = None,
                      units: Optional[int] = None):
     """Dense tensor-core scoring + mask + top-k (pc_score_topk_dense).  Returns (scores f64 [R,k], idx i64 [R,k],
-    flags i32 [R]); flagged rows must be re-run on the exact path (topk_segments)."""
+    flags i32 [R]); flagged rows must be re-run on the exact path (topk_by_type)."""
     q = q.contiguous()
     rows, dim = q.shape
     if max_norm is None:

@@ -241,6 +241,12 @@ class CatalogIndex:
             self.members, self.offsets = csr.col, csr.rowptr
             self.num_types = n_types
 
+    def _whole_run(self) -> torch.Tensor:
+        """type_offsets {0, P} of one type holding the whole catalog: the run of rows without a row type."""
+        if self._all is None:
+            self._all = torch.tensor([0, self.num_products], dtype=torch.int64, device=self.catalog.device)
+        return self._all
+
     def topk(self, queries: torch.Tensor, k: int, row_type: Optional[torch.Tensor] = None,
              splits: Optional[int] = None, exclude: Optional[Exclusions] = None) -> Tuple[torch.Tensor, torch.Tensor]:
         """Top-k per query row, 1 <= k <= ops.TOPK_MAX_K (1024; ValueError otherwise); row_type[r] restricts row r
@@ -250,9 +256,8 @@ class CatalogIndex:
         queries = queries.contiguous().float()
         _check_exclusions(exclude, queries.shape[0], "CatalogIndex.topk")
         if row_type is None:
-            if self._all is None:
-                self._all = torch.tensor([0, self.num_products], dtype=torch.int64, device=queries.device)
-            return ops.topk_by_type(queries, self.catalog, self._all, 1, None, k, None, self.index_base, splits, exclude)
+            return ops.topk_by_type(queries, self.catalog, self._whole_run(), 1, None, k, None, self.index_base, splits,
+                                    exclude)
         if self.offsets is None:
             raise ValueError("CatalogIndex.topk: the catalog was built without type ids")
         rt = row_type.to(queries.device, torch.int32).contiguous()
@@ -304,10 +309,8 @@ class CatalogIndex:
         if self.num_products == 0:
             return torch.zeros(queries.shape[0], dtype=torch.int64, device=queries.device)
         if row_type is None:
-            if self._all is None:
-                self._all = torch.tensor([0, self.num_products], dtype=torch.int64, device=queries.device)
-            return ops.rank_by_type(queries, self.catalog, self._all, 1, None, target_rows, targets, None, self.index_base,
-                                    splits, exclude)
+            return ops.rank_by_type(queries, self.catalog, self._whole_run(), 1, None, target_rows, targets, None,
+                                    self.index_base, splits, exclude)
         return ops.rank_by_type(queries, self.catalog, self.offsets, self.num_types, row_type, target_rows, targets,
                                 self.members, self.index_base, splits, exclude, self.type_id)
 
