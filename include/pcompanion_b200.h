@@ -200,6 +200,22 @@ int pc_hinge_type_bwd(const float* sims, const int64_t* pos, const int64_t* neg,
  * Reproducible from (seed, batch slot). */
 int pc_sample_negatives(const int32_t* anchor, const int64_t* sim_rowptr, const int32_t* sim_col, int64_t batch,
                         int32_t n_nodes, int k, uint64_t seed, int32_t* out, pc_stream_t stream);
+/* Feature rows of one triplet batch in one launch (data_loader.py:27-88,171-206 and the three forward calls of
+ * product2vec.py:132-134, without collate_fn's zero padding).  table [N, dim] with row stride ld (floats), anchor and
+ * positive int64 [batch], negatives int64 [batch, kneg], the co-view CSR (rowptr int64 [N + 1], col int32) and
+ * nbr_ptr int64 [batch + 1], the exclusive prefix sum of the anchors' co-view degrees (nbr_ptr[0] = 0,
+ * nbr_ptr[batch] = n_nbr; the caller computes it).  Writes
+ *   rows float [batch + n_nbr + batch + batch * kneg, dim] = anchors | neighbour rows | positives | negatives,
+ *     anchor b's neighbours at rows batch + nbr_ptr[b] .. in ascending CSR order (collate_fn's order);
+ *   edge_row int32 [n_nbr]: the batch slot of every neighbour row, i.e. the CSC row list of the batch graph
+ *     (row b attends to neighbour rows nbr_ptr[b] .. nbr_ptr[b + 1]).
+ * One warp per anchor, 16-byte copies.  dim % 4 == 0, dim <= 1024, ld % 4 == 0, table and rows 16-byte aligned,
+ * batch and n_nbr < 2^31, kneg >= 1; col / edge_row may be NULL when n_nbr == 0.  Indices are not checked: an anchor,
+ * positive or negative outside [0, N), or an nbr_ptr that is not the prefix sum of the anchors' degrees, is undefined
+ * behaviour (as for pc_sample_negatives and pc_rows_gather). */
+int pc_triplet_batch_rows(const float* table, int64_t ld, int dim, const int64_t* anchor, const int64_t* positive,
+                          const int64_t* negatives, int64_t batch, int kneg, const int64_t* rowptr, const int32_t* col,
+                          const int64_t* nbr_ptr, int64_t n_nbr, float* rows, int32_t* edge_row, pc_stream_t stream);
 
 /* ------------------------------------------------------------------ (4) retrieval
  * Replaces torch.matmul + torch.topk of p_companion.py:60-64, metrics.py:21,89 and the

@@ -11,10 +11,10 @@ from .bpg import BehaviorProductGraph
 from .p_companion import ComplementaryItemPrediction, ComplementaryTypeTransition, PCompanion
 from .product2vec import Product2Vec
 from .retrieval import CatalogIndex, Exclusions, Metrics, ShardedCatalog
-from .data import ComplementaryDataset, GraphTripletSampler, SimilarityDataset, collate_fn
+from .data import ComplementaryDataset, GraphTripletSampler, SimilarityDataset, TripletBatch, collate_fn
 from .inference import PCompanionInference
 from .graphs import GraphedTrainStep
 
 __all__ = ["ops", "BehaviorProductGraph", "Product2Vec", "ComplementaryTypeTransition",
            "ComplementaryItemPrediction", "PCompanion", "Metrics", "CatalogIndex", "Exclusions", "ShardedCatalog",
-           "SimilarityDataset", "ComplementaryDataset", "collate_fn", "GraphTripletSampler", "PCompanionInference", "GraphedTrainStep"]
+           "SimilarityDataset", "ComplementaryDataset", "collate_fn", "GraphTripletSampler", "TripletBatch", "PCompanionInference", "GraphedTrainStep"]

@@ -59,6 +59,7 @@ PROTOTYPES = {
     "pc_hinge_type_fwd": (c_int, [P, P, P, c_int64, c_int64, c_float, P, P, P]),
     "pc_hinge_type_bwd": (c_int, [P, P, P, c_int64, c_int64, c_float, P, P, P]),
     "pc_sample_negatives": (c_int, [P, P, P, c_int64, ctypes.c_int32, c_int, c_uint64, P, P]),
+    "pc_triplet_batch_rows": (c_int, [P, c_int64, c_int, P, P, P, c_int64, c_int, P, P, P, c_int64, P, P, P]),
     "pc_topk_groups_workspace_bytes": (c_size_t, [c_int64, c_int, c_int]),
     "pc_topk_groups": (c_int, [P, c_int64, c_int, P, P, P, P, P, P, c_int64, c_int, c_int, c_int64, P, P, P, c_size_t, P]),
     "pc_topk_by_type_workspace_bytes": (c_size_t, [c_int64, c_int, c_int]),

@@ -10,14 +10,15 @@ Two layers:
 * ``GraphTripletSampler``: the CSR-native path.  A batch is a few index tensors on the device
   (anchor, positive, negatives) into the full-graph embedding table; negatives come from
   pcompanion_b200/csrc/sample.cu (same rejection rule as data_loader.py:27-40).  No feature copies,
-  no padding, no Python per sample.
+  no padding, no Python per sample.  ``neighborhood_batches`` / ``TripletBatch`` add each anchor's co-view
+  neighbour offsets for the reference's mini-batch step (Product2Vec.triplet_loss_graph).
 """
 from __future__ import annotations
 
 import logging
 import random
 from collections import defaultdict
-from typing import Dict, List, Optional, Tuple
+from typing import Dict, List, NamedTuple, Optional, Tuple
 
 import torch
 from torch.utils.data import Dataset
@@ -221,3 +222,46 @@ class GraphTripletSampler:
             pick = perm[i: i + batch_size]
             a, p = self.anchor[pick], self.positive[pick]
             yield a.to(torch.int64), p.to(torch.int64), self.negatives_for(a, seed * 1_000_003 + i).to(torch.int64)
+
+    def neighborhood_batches(self, batch_size: int, seed: int, csr: ops.CSRGraph):
+        """epoch(batch_size, seed)'s triplets (same order, same negatives) as TripletBatch with each anchor's co-view
+        neighbour offsets into `csr` (Product2Vec.triplet_loss_graph).  The anchors' degrees are taken in permutation order
+        and summed once for the whole epoch; every batch's neighbour total comes back to the host in ONE read, before the
+        first batch, so no batch of a graph without hub rows synchronises (ops.triplet_batch_rows)."""
+        self._require_k()
+        if csr.n_rows != self.num_nodes:
+            raise ValueError(f"neighborhood_batches: the CSR has {csr.n_rows} rows for {self.num_nodes} products")
+        g = torch.Generator(device=self.device).manual_seed(int(seed))
+        perm = torch.randperm(len(self), generator=g, device=self.device)
+        anchors = self.anchor[perm].to(torch.int64)
+        cum = torch.zeros(len(self) + 1, dtype=torch.int64, device=self.device)
+        cum[1:] = torch.cumsum(csr.rowptr[anchors + 1] - csr.rowptr[anchors], 0)
+        starts = range(0, len(self), batch_size)
+        bounds = torch.cat([cum[:-1:batch_size], cum[-1:]])
+        totals = (bounds[1:] - bounds[:-1]).tolist()                       # the epoch's one host read
+        csr.hub_split()               # whether batch graphs split hub rows: one read per graph, cached on the CSR
+        for i, n_nbr in zip(starts, totals):
+            a = anchors[i: i + batch_size]
+            yield TripletBatch(a, self.positive[perm[i: i + batch_size]].to(torch.int64),
+                               self.negatives_for(a, seed * 1_000_003 + i).to(torch.int64),
+                               cum[i: i + a.numel() + 1] - cum[i], n_nbr)
+
+
+class TripletBatch(NamedTuple):
+    """One graph-native triplet batch: int64 index tensors on the device - anchor [B], positive [B], negatives [B, K] -
+    and nbr_ptr int64 [B + 1], the prefix sum of the anchors' co-view degrees, with n_nbr = nbr_ptr[B] on the host."""
+    anchor: torch.Tensor
+    positive: torch.Tensor
+    negatives: torch.Tensor
+    nbr_ptr: torch.Tensor
+    n_nbr: int
+
+    @classmethod
+    def build(cls, csr: ops.CSRGraph, anchor: torch.Tensor, positive: torch.Tensor, negatives: torch.Tensor) -> "TripletBatch":
+        """A batch of caller-chosen triplets (one host read: the neighbour total)."""
+        anchor = anchor.reshape(-1).to(csr.rowptr.device, torch.int64).contiguous()
+        positive = positive.reshape(-1).to(anchor.device, torch.int64).contiguous()
+        negatives = negatives.reshape(anchor.numel(), -1).to(anchor.device, torch.int64).contiguous()
+        nbr_ptr = torch.zeros(anchor.numel() + 1, dtype=torch.int64, device=anchor.device)
+        nbr_ptr[1:] = torch.cumsum(csr.rowptr[anchor + 1] - csr.rowptr[anchor], 0)
+        return cls(anchor, positive, negatives, nbr_ptr, int(nbr_ptr[-1].item()))

@@ -235,6 +235,35 @@ def regular_graph(batch: int, n_nbr: int, device) -> CSRGraph:
     return g
 
 
+def triplet_batch_rows(table: torch.Tensor, csr: CSRGraph, anchor: torch.Tensor, positive: torch.Tensor,
+                       negatives: torch.Tensor, nbr_ptr: torch.Tensor, n_nbr: int):
+    """Feature rows of one triplet batch in one launch (pc_triplet_batch_rows): returns (anchor_rows [B, D],
+    neighbour_rows [n_nbr, D], positive_rows [B, D], negative_rows [B * kneg, D]), contiguous views of one buffer, and
+    the batch graph: row b attends to neighbour rows nbr_ptr[b] .. nbr_ptr[b + 1] (anchor b's co-view neighbours in CSR
+    order), with its transpose filled in.  nbr_ptr int64 [B + 1] is the prefix sum of the anchors' co-view degrees and
+    n_nbr == nbr_ptr[B] its host copy (GraphTripletSampler.neighborhood_batches / TripletBatch.build).
+
+    The batch graph splits hub rows only when the full CSR has any (csr.hub_split(), one host read per graph); it then
+    takes one host read per batch to find its own hub rows.  A graph without hubs reads nothing back per batch."""
+    b = anchor.numel()
+    if table.dim() != 2 or positive.numel() != b or negatives.dim() != 2 or negatives.shape[0] != b or nbr_ptr.numel() != b + 1:
+        raise ValueError(f"triplet_batch_rows: table [N, D], anchor [B], positive [B], negatives [B, K] and nbr_ptr [B + 1] "
+                         f"expected, got {tuple(table.shape)}, {tuple(anchor.shape)}, {tuple(positive.shape)}, "
+                         f"{tuple(negatives.shape)}, {tuple(nbr_ptr.shape)}")
+    kneg, d, n_nbr = negatives.shape[1], table.shape[1], int(n_nbr)
+    rows = torch.empty(2 * b + n_nbr + b * kneg, d, dtype=F32, device=table.device)
+    edge_row = torch.empty(n_nbr, dtype=I32, device=table.device)
+    call("pc_triplet_batch_rows", _f32_cuda(table, "table"), table.stride(0), d, dev(anchor, I64, "anchor"),
+         dev(positive, I64, "positive"), dev(negatives, I64, "negatives"), b, kneg, dev(csr.rowptr, I64, "rowptr"),
+         dev(csr.col, I32, "col"), dev(nbr_ptr, I64, "nbr_ptr"), n_nbr, dev(rows, F32, "rows"), dev(edge_row, I32, "edge_row"),
+         stream())
+    a_rows, nbr_rows, p_rows, n_rows = rows.split([b, n_nbr, b, b * kneg])
+    graph = CSRGraph(nbr_ptr, torch.arange(n_nbr, dtype=I32, device=table.device), b, n_nbr,
+                     (torch.arange(n_nbr + 1, dtype=I64, device=table.device), edge_row),
+                     split_hubs=csr.hub_split() is not None, _hub_t=(None,))   # every neighbour row has one edge: no hub columns
+    return a_rows, nbr_rows, p_rows, n_rows, graph
+
+
 # --------------------------------------------------------------------------- GAT
 def _f32_cuda(t: torch.Tensor, what: str):
     if not t.is_cuda or t.dtype != F32 or t.stride(-1) != 1:

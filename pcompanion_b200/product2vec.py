@@ -11,7 +11,10 @@ called - the attention core runs in pcompanion_b200/csrc/gat.cu over a CSR:
   as a regular CSR (row i -> rows i*N..(i+1)*N), so zero-padded rows are attended exactly as the
   reference does (no key_padding_mask, SURVEY fact 3) and BatchNorm sees the same B*N rows;
 * graph API ``forward_graph(x, csr)``: FFN and K|V projection once per node, attention over the
-  BPG's co-view CSR (the formulation that scales to 200 M edges, SURVEY H2).
+  BPG's co-view CSR (the formulation that scales to 200 M edges, SURVEY H2);
+* graph-native training ``triplet_loss_graph`` / ``train_model_graph``: the reference's mini-batch step
+  (four FFN calls with their own BatchNorm statistics, attention for the anchors only) on rows gathered
+  on the device from index tensors - no host feature copies, no padding, no Python per sample.
 """
 from __future__ import annotations
 
@@ -160,6 +163,55 @@ class Product2Vec(nn.Module):
         """Same loss on rows of a full-graph embedding table picked by index (graph training: the batch is index
         tensors into forward_graph's output instead of padded feature copies, SURVEY 8f.1)."""
         return ops.triplet_hinge_indexed(table, anchor_idx, positive_idx, negative_idx, self.config.MARGIN)
+
+    def triplet_loss_graph(self, x: torch.Tensor, csr: ops.CSRGraph, batch) -> torch.Tensor:
+        """The loss of one training batch of product2vec.py:132-154 from index tensors (a data.TripletBatch) into the
+        feature table x [N, D] and its co-view CSR.  The rows are gathered on the device in one launch, then the four FFN
+        calls run in the reference's order - anchors, neighbour rows, positives, negatives - each with the batch statistics
+        of its own rows and its own running-statistics update.  Anchors attend over exactly their co-view neighbours;
+        anchors without any keep ffn(x) (forward_graph, generate_all_embeddings), and a batch without neighbour rows
+        skips the neighbour FFN and the attention.  Unlike the drop-in path there are no zero-padding rows: the two agree
+        bit for bit when every anchor of the batch has the same degree >= 1.  x is not differentiated."""
+        _require_cuda(x, "triplet_loss_graph")
+        a_rows, nbr_rows, p_rows, n_rows, graph = ops.triplet_batch_rows(
+            x, csr, batch.anchor, batch.positive, batch.negatives, batch.nbr_ptr, batch.n_nbr)
+        anchor_emb = self._ffn_rows(a_rows)
+        if batch.n_nbr > 0:
+            out = self._attend(anchor_emb, self._ffn_rows(nbr_rows), graph)
+            has_nbr = (batch.nbr_ptr[1:] > batch.nbr_ptr[:-1]).unsqueeze(1)
+            anchor_emb = torch.where(has_nbr, out, anchor_emb)
+        positive_emb = self._ffn_rows(p_rows)
+        negative_emb = self._ffn_rows(n_rows).view(batch.negatives.shape[0], batch.negatives.shape[1], -1)
+        return self.triplet_loss(anchor_emb, positive_emb, negative_emb)
+
+    def train_model_graph(self, bpg, optimizer, num_epochs=10, batch_size=None, seed=0, k_neg=5) -> Dict[str, torch.Tensor]:
+        """train_model's loop without the host data path: batches come from GraphTripletSampler.neighborhood_batches
+        over the BPG's similarity pairs (epoch e uses seed * 100_003 + e), each step is triplet_loss_graph, and the loss is
+        summed on the device (one host read per epoch for the log line, one for the epoch's plan).  Same log line and
+        return value as train_model.  batch_size defaults to config.BATCH_SIZE."""
+        from .data import GraphTripletSampler
+        device = self.config.DEVICE
+        logger = logging.getLogger(__name__)
+        self.to(device)
+        bpg.finalize()
+        sampler = GraphTripletSampler(bpg, k_neg=k_neg)
+        csr = bpg.csr("co_view")
+        x = bpg.features.to(device)
+        batch_size = self.config.BATCH_SIZE if batch_size is None else int(batch_size)
+        for epoch in range(num_epochs):
+            self.train()
+            total_loss = torch.zeros((), dtype=torch.float32, device=device)
+            num_batches = 0
+            for batch in sampler.neighborhood_batches(batch_size, seed * 100_003 + epoch, csr):
+                loss = self.triplet_loss_graph(x, csr, batch)
+                optimizer.zero_grad()
+                loss.backward()
+                optimizer.step()
+                total_loss += loss.detach()
+                num_batches += 1
+            logger.info(f"Epoch {epoch + 1}/{num_epochs}, Loss: {total_loss.item() / max(num_batches, 1):.4f}")
+        self.eval()
+        return self.generate_all_embeddings(bpg)
 
     def train_model(self, train_loader, optimizer, num_epochs=10) -> Dict[str, torch.Tensor]:
         """Training loop of product2vec.py:113-170 (same batch keys, same return value)."""
