@@ -265,14 +265,25 @@ class CatalogIndex:
                                 splits, exclude)
 
     def topk_dense(self, queries: torch.Tensor, k: int, row_type: Optional[torch.Tensor] = None):
-        """Same result as ``topk`` through the dense tensor-core path (BASELINE north_star part 4): single-pass TF32 scoring
-        GEMM over the whole catalog, per-type mask and candidate selection in the epilogue, exact fp64 re-scoring.
-        Rows whose guard band fails are re-run on the exact segmented kernel, so the output is always exact."""
+        """Same result as ``topk`` (bit for bit, every row type) through the dense tensor-core path (BASELINE north_star
+        part 4): single-pass TF32 scoring GEMM over the whole catalog, per-type mask and candidate selection in the
+        epilogue, exact fp64 re-scoring.  Rows whose guard band fails are re-run on the exact segmented kernel, so the
+        output is always exact.  1 <= k <= 16 and D in {32, 64, 96, 128} (RuntimeError otherwise).  As in ``topk``, a
+        row type outside [0, num_types) gives (-inf, -1) padding, and row types on a catalog built without type ids
+        raise ValueError."""
         queries = queries.contiguous().float()
+        if row_type is not None and self.type_id is None:
+            raise ValueError("CatalogIndex.topk_dense: the catalog was built without type ids")
         if self._max_norm is None:
             self._max_norm = float(self.catalog.norm(dim=1).max().item())
         rt = None if row_type is None else row_type.to(queries.device, torch.int32).contiguous()
         s, i, flags = ops.score_topk_dense(queries, self.catalog, k, self.type_id, rt, self.index_base, self._max_norm)
+        if rt is not None:
+            # the kernel reads a negative row type as "no restriction"; topk lists nothing outside [0, num_types)
+            out = ((rt < 0) | (rt >= self.num_types)).unsqueeze(1)
+            s.masked_fill_(out, float("-inf"))
+            i.masked_fill_(out, -1)
+            flags.masked_fill_(out.squeeze(1), 0)
         bad = torch.nonzero(flags).squeeze(1)
         if bad.numel():
             fs, fi = self.topk(queries[bad], k, None if rt is None else rt[bad])
